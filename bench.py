@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native frame-synthesis hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload adacof|pipeline] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload adacof|pipeline] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by the driver as
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
@@ -31,6 +31,25 @@ for p in (ROOT, PKG):
 
 METRIC = "interpolated_1080p_frames_per_s"
 UNIT = "frames/s"
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(outputs, path, seed=0):
+    """Writes each output of the last timed step as path/<name>.npy (float32).  Outputs of more than DUMP_BYTES in all are
+    sampled: the same fraction of every array, flattened, at element indices drawn from a generator seeded with ``seed``, so
+    runs with the same arguments store the same elements and two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = sum(t.numel() for t in outputs.values())
+    keep = (DUMP_BYTES - 4096 * len(outputs)) // 4          # float32 elements, less room for the .npy headers
+    rng = np.random.default_rng(seed)
+    for name, t in outputs.items():
+        t = t.detach()
+        if total > keep:
+            idx = np.sort(rng.integers(0, t.numel(), t.numel() * keep // total))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
 
 
 def measured_peaks():
@@ -137,6 +156,11 @@ class AdaCoFWorkload:
         if timed:
             e[2].record()
             self.ev.append(e)
+
+    def outputs(self):
+        """What a caller of the timed step receives: the warped frames and the three coefficient gradients."""
+        _, gw, gi, gj = self.grads
+        return {"out": self.out, "grad_weight": gw, "grad_offset_i": gi, "grad_offset_j": gj}
 
     def roofline(self, peak, peak_src):
         fwd = sum(e[0].elapsed_time(e[1]) for e in self.ev) / len(self.ev)
@@ -300,8 +324,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-refbar", action="store_true", help="skip timing the reference's own CUDA kernels")
     ap.add_argument("--no-records", action="store_true", help="N > 1: skip the configs[4] training / configs[3] 4K records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) to DIR/<name>.npy, float32; above %d MB in all, the "
+                         "same seeded sample of each output" % (DUMP_BYTES // 10 ** 6))
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "fvfi":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl fvfi)")
 
     if args.impl == "reference":
         return run_reference(args, emit)
@@ -347,6 +378,8 @@ def main():
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_per_step = float(ms.item()) / args.steps
     value = wl.frames_per_step * world / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl.outputs(), args.dump_outputs)      # before anything below runs the workload again
 
     line = None
     if rank == 0:

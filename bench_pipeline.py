@@ -66,6 +66,10 @@ class PipelineWorkload:
             self._pending.append(self.pipe.timing)
             self.pipe.timing = None
 
+    def outputs(self):
+        """What a caller of the timed step receives: the interpolated frames."""
+        return {"frame": self.out}
+
     def _collect(self):
         for tl in getattr(self, "_pending", []):
             for (n0, e0), (n1, e1) in zip(tl[:-1], tl[1:]):

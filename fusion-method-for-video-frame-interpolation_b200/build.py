@@ -27,7 +27,8 @@ def stale():
     if not os.path.exists(OUT):
         return True
     t = os.path.getmtime(OUT)
-    deps = sources() + glob.glob(os.path.join(HERE, "csrc", "*.cuh")) + glob.glob(os.path.join(ROOT, "include", "*.h"))
+    deps = sources() + glob.glob(os.path.join(HERE, "csrc", "*.cuh")) + glob.glob(os.path.join(HERE, "csrc", "*.hpp"))
+    deps += glob.glob(os.path.join(ROOT, "include", "*.h"))
     deps.append(os.path.abspath(__file__))
     return any(os.path.getmtime(d) > t for d in deps)
 

@@ -4,8 +4,7 @@ Imports the reference's own Python modules from /root/reference (present only
 in the build container, never on the GPU box) with empty stubs for its missing
 third-party dependencies (SURVEY.md Appendix F).  Used by
   * oracle/build_ref_kernels.py   (expands + compiles the reference CUDA kernels)
-  * tests/golden/make_golden.py   (generates the committed golden fixtures)
-  * tests marked `needs_reference` (skipped when /root/reference is absent).
+  * tests/golden/make_golden*.py  (generate the committed golden fixtures the tests compare against).
 Nothing here is copied from the reference; it is imported where it lies.
 """
 import os

@@ -14,19 +14,14 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
     has_gpu = torch.cuda.is_available()
-    from oracle import ref_import
-    has_ref = ref_import.available()
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "needs_reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 @pytest.fixture(scope="session")

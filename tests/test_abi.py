@@ -83,28 +83,22 @@ def test_state_dict_keys_match_reference_checkpoints():
     assert "get_kernel.moduleConv1.0.weight" in an.state_dict() and "get_kernel.moduleOcclusion.7.bias" in an.state_dict()
 
 
-@pytest.mark.needs_reference
-def test_state_dicts_load_into_reference_modules():
-    """The mirrors' state_dicts load into the REAL reference modules and vice versa (strict)."""
+def test_state_dicts_load_into_reference_modules(golden_dir):
+    """The mirrors' state_dicts have exactly the keys and shapes of the REAL reference modules: the state the reference's own
+    PhaseNet / FusionNet loaded strictly to make the committed pipeline fixtures (tests/golden/make_golden_models.py; the
+    fixture's checksum pins it) loads strictly into the mirrors, so either side's state_dict loads into the other."""
     import types
     import numpy as np
     import torch
-    from oracle import ref_import
-    ref_import.install_stubs()
-    from src.fusion_net.fusion_net import FusionNet as RefFusion
-    from src.phase_net.phase_net import PhaseNet as RefPhase
-    from src.train.pyramid import Pyramid as RefPyramid
     from fvfi.fusion_net import FusionNet
     from fvfi.phase_net import PhaseNet
-    cpu = torch.device("cpu")
-    rp = RefPhase(RefPyramid(12, 4, np.sqrt(2), cpu), cpu, 2)
-    PhaseNet(types.SimpleNamespace(height=12, nbands=4), cpu, 2).load_state_dict(rp.state_dict(), strict=True)
-    RefFusion().load_state_dict(FusionNet().state_dict(), strict=True)
-    for name in ("src/phase_net/phase_net.pt", "src/fusion_net/fusion_net.pt"):
-        path = os.path.join(ref_import.REF, name)
-        if os.path.exists(path) and os.path.getsize(path) > 10000:
-            sd = torch.load(path, map_location="cpu")
-            (PhaseNet(types.SimpleNamespace(height=12, nbands=4), cpu, 2) if "phase" in name else FusionNet()).load_state_dict(sd, strict=True)
+    from oracle import fusion_pipeline as fp
+    z = np.load(os.path.join(golden_dir, "pipeline_ref_B1_64x64_s0.npz"))
+    state = fp.seeded_state(int(z["meta"][3]))
+    chk = [float(sum(v.double().sum() for v in state[n].values())) for n in ("phase_net", "fusion_net", "adacof")]
+    assert np.allclose(chk, z["checksum"], rtol=1e-9), "seeded init differs from the fixture's"
+    PhaseNet(types.SimpleNamespace(height=12, nbands=4), torch.device("cpu"), 2).load_state_dict(state["phase_net"], strict=True)
+    FusionNet().load_state_dict(state["fusion_net"], strict=True)
 
 
 def test_backward_entry_points_validate_arguments():
