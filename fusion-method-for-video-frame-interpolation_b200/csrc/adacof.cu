@@ -450,13 +450,29 @@ adacofnet_warp_blend_direct(const float* __restrict__ in1, const float* __restri
     if (mask) mask[(size_t)n * plane + p] = fminf(fmaxf(fmaxf(var[0], var[1]), 0.f), 20.f) / 20.f;
 }
 
+__device__ __forceinline__ float fusion_blend_px(float base, float x) {
+    const float v = base + tanhf(x);                              // fusion_net.py:67-72
+    return fminf(fmaxf(v, 0.f), 1.f);                             // fusion_net.py:77
+}
+
 __global__ void fusion_blend_kernel(const float* __restrict__ base, const float* __restrict__ x,
                                     float* __restrict__ out, size_t n) {
     const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) {
-        const float v = base[t] + tanhf(x[t]);                    // fusion_net.py:67-72
-        out[t] = fminf(fmaxf(v, 0.f), 1.f);                       // fusion_net.py:77
-    }
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += stride) out[t] = fusion_blend_px(base[t], x[t]);
+}
+
+// The same blend for frames that leave as 8-bit video: planar [B,3,H,W] in, interleaved rgb24 [B,H,W,3] out, rint(v * 255) (round
+// half to even); the fp32 frame is never stored.
+__global__ void __launch_bounds__(256) fusion_blend_rgb8_kernel(const float* __restrict__ base, const float* __restrict__ x,
+                                                                uint8_t* __restrict__ out, size_t plane) {
+    const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = blockIdx.y;
+    if (p >= plane) return;
+    const size_t o = (size_t)n * 3 * plane + p;
+    uint8_t* dst = out + ((size_t)n * plane + p) * 3;
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+        dst[c] = (uint8_t)__float2uint_rn(fusion_blend_px(__ldcs(base + o + c * plane), __ldcs(x + o + c * plane)) * 255.f);
 }
 
 static int check_dims(int B, int C, int Hin, int Win, int H, int W, int F, int dil) {
@@ -647,6 +663,16 @@ extern "C" int fvfi_fusion_blend(const float* base, const float* x_pre_tanh, flo
     size_t blocks = (n + 255) / 256;
     if (blocks > (size_t)sms * 16) blocks = (size_t)sms * 16;
     fusion_blend_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(base, x_pre_tanh, out, n);
+    FVFI_LAUNCH_CHECK();
+    return FVFI_OK;
+}
+
+extern "C" int fvfi_fusion_blend_rgb8(const float* base, const float* x_pre_tanh, uint8_t* out, int B, int H, int W, void* stream) {
+    FVFI_CHECK_ARG(base && x_pre_tanh && out, "fvfi_fusion_blend_rgb8: null pointer");
+    FVFI_CHECK_ARG(B > 0 && H > 0 && W > 0 && B <= 65535, "fvfi_fusion_blend_rgb8: bad size B=%d H=%d W=%d", B, H, W);
+    const size_t plane = (size_t)H * W;
+    dim3 grid((unsigned)((plane + 255) / 256), B);
+    fusion_blend_rgb8_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(base, x_pre_tanh, out, plane);
     FVFI_LAUNCH_CHECK();
     return FVFI_OK;
 }

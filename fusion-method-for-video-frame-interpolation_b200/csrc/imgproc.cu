@@ -18,21 +18,43 @@ __device__ __forceinline__ float lin_to_srgb(float c) {
 __device__ __forceinline__ float lab_f(float t) { return t > 0.008856f ? cbrtf(t) : 7.787f * t + 16.f / 116.f; }
 __device__ __forceinline__ float lab_finv(float f) { return f > 0.2068966f ? f * f * f : (f - 16.f / 116.f) / 7.787f; }
 
+// One pixel: sRGB in [0,1] -> scaled Lab written at dst[0], dst[plane], dst[2*plane] (shared by rgb2lab_kernel and
+// rgb8_to_rgb_lab_kernel, so both give the same bits for the same RGB value).
+__device__ __forceinline__ void rgb_to_scaled_lab(float sr, float sg, float sb, float* dst, size_t plane) {
+    const float r = srgb_to_lin(sr), g = srgb_to_lin(sg), b = srgb_to_lin(sb);
+    const float x = (0.412453f * r + 0.357580f * g + 0.180423f * b) / 0.95047f;
+    const float y = (0.212671f * r + 0.715160f * g + 0.072169f * b);
+    const float z = (0.019334f * r + 0.119193f * g + 0.950227f * b) / 1.08883f;
+    const float fx = lab_f(x), fy = lab_f(y), fz = lab_f(z);
+    dst[0] = (116.f * fy - 16.f) / 100.f;                    // transform.py:9  L / light
+    dst[plane] = (500.f * (fx - fy) + 128.f) / 255.f;        // transform.py:10-11
+    dst[2 * plane] = (200.f * (fy - fz) + 128.f) / 255.f;
+}
+
 __global__ void rgb2lab_kernel(const float* __restrict__ rgb, float* __restrict__ lab, size_t plane, int B) {
     const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int n = blockIdx.y;
     if (p >= plane) return;
     const float* src = rgb + (size_t)n * 3 * plane + p;
-    const float r = srgb_to_lin(src[0]), g = srgb_to_lin(src[plane]), b = srgb_to_lin(src[2 * plane]);
-    const float x = (0.412453f * r + 0.357580f * g + 0.180423f * b) / 0.95047f;
-    const float y = (0.212671f * r + 0.715160f * g + 0.072169f * b);
-    const float z = (0.019334f * r + 0.119193f * g + 0.950227f * b) / 1.08883f;
-    const float fx = lab_f(x), fy = lab_f(y), fz = lab_f(z);
-    float* dst = lab + (size_t)n * 3 * plane + p;
-    dst[0] = (116.f * fy - 16.f) / 100.f;                    // transform.py:9  L / light
-    dst[plane] = (500.f * (fx - fy) + 128.f) / 255.f;        // transform.py:10-11
-    dst[2 * plane] = (200.f * (fy - fz) + 128.f) / 255.f;
+    rgb_to_scaled_lab(src[0], src[plane], src[2 * plane], lab + (size_t)n * 3 * plane + p, plane);
     (void)B;
+}
+
+// Decoder frames [T,H,W,3] uint8 (interleaved rgb24) -> planar fp32 RGB [T,3,H,W] (k / 255, correctly rounded: __fdiv_rn, not a
+// reciprocal multiply) and planar scaled Lab [T,3,H,W] in one pass.  A warp reads 96 contiguous bytes and writes coalesced planes.
+__global__ void __launch_bounds__(256) rgb8_to_rgb_lab_kernel(const uint8_t* __restrict__ rgb8, float* __restrict__ rgb,
+                                                              float* __restrict__ lab, size_t plane) {
+    const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = blockIdx.y;
+    if (p >= plane) return;
+    const uint8_t* src = rgb8 + ((size_t)n * plane + p) * 3;
+    const float r = __fdiv_rn((float)__ldg(src), 255.f), g = __fdiv_rn((float)__ldg(src + 1), 255.f),
+                b = __fdiv_rn((float)__ldg(src + 2), 255.f);
+    const size_t o = (size_t)n * 3 * plane + p;
+    rgb[o] = r;
+    rgb[o + plane] = g;
+    rgb[o + 2 * plane] = b;
+    rgb_to_scaled_lab(r, g, b, lab + o, plane);
 }
 
 __global__ void lab2rgb_kernel(const float* __restrict__ lab, float* __restrict__ rgb, size_t plane, int B) {
@@ -415,6 +437,16 @@ extern "C" int fvfi_rgb2lab(const float* rgb, float* lab, int B, int H, int W, v
     return FVFI_OK;
 }
 
+extern "C" int fvfi_rgb8_to_rgb_lab(const uint8_t* rgb8, float* rgb, float* lab, int T, int H, int W, void* stream) {
+    FVFI_CHECK_ARG(rgb8 && rgb && lab, "fvfi_rgb8_to_rgb_lab: null pointer");
+    FVFI_CHECK_ARG(T > 0 && H > 0 && W > 0 && T <= 65535, "fvfi_rgb8_to_rgb_lab: bad size T=%d H=%d W=%d", T, H, W);
+    const size_t plane = (size_t)H * W;
+    dim3 grid((unsigned)((plane + 255) / 256), T);
+    rgb8_to_rgb_lab_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rgb8, rgb, lab, plane);
+    FVFI_LAUNCH_CHECK();
+    return FVFI_OK;
+}
+
 extern "C" int fvfi_lab2rgb(const float* lab, float* rgb, int B, int H, int W, void* stream) {
     FVFI_CHECK_ARG(rgb && lab && B > 0 && H > 0 && W > 0 && B <= 65535, "lab2rgb: bad argument");
     const size_t plane = (size_t)H * W;
@@ -606,21 +638,22 @@ __global__ void __launch_bounds__(256) nchw_to_nhwc_slice_kernel(const float* __
 }
 
 // ---- PhaseNet glue (src/train/utils.py:47-127, src/phase_net/phase_net.py:42-105,141,155-156) --------------------------------
-// Input side: the decomposition of [frame-1 planes | frame-2 planes] (N = 2*P planes, channel = plane*nb + band) goes straight
+// Input side: the decomposition of the frames (channel = plane*nb + band; frame 2 of pair-plane p is plane p + q: q = P for
+// [frame-1 planes | frame-2 planes], q = 3 for a clip of consecutive frames decomposed once) goes straight
 // into the 4*nb value channels of the NHWC concat of planes [p0, p0+pc):  [phase_1 | phase_2] / pi,  [amp_1 | amp_2] / den[p]
 // (den = per-plane max over both frames + eps, from the decomposition's own epilogue) -- separate_vals, get_concat_layers_inf,
 // normalize_vals and the concat in ONE pass over the planes (the reference materialises each of them).
 template <int NB>
 __global__ void __launch_bounds__(256) phasenet_assemble_kernel(const float* __restrict__ phase, const float* __restrict__ amp,
                                                                 const float* __restrict__ den, float* __restrict__ y, size_t plane,
-                                                                int ldy, int P, int p0) {
+                                                                int ldy, int q, int p0) {
     const size_t px = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (px >= plane) return;
     const int p = p0 + blockIdx.y;
     const float* ph1 = phase + (size_t)p * NB * plane + px;
-    const float* ph2 = phase + (size_t)(P + p) * NB * plane + px;
+    const float* ph2 = phase + (size_t)(q + p) * NB * plane + px;
     const float* am1 = amp + (size_t)p * NB * plane + px;
-    const float* am2 = amp + (size_t)(P + p) * NB * plane + px;
+    const float* am2 = amp + (size_t)(q + p) * NB * plane + px;
     const float d = __ldg(den + p);
     float v[4 * NB];
 #pragma unroll
@@ -647,7 +680,7 @@ __global__ void __launch_bounds__(256) phasenet_assemble_kernel(const float* __r
 template <int NB>
 __global__ void __launch_bounds__(256) phasenet_outputs_kernel(const float* __restrict__ pred, int ldp, const float* __restrict__ amp,
                                                                float* __restrict__ phase_out, float* __restrict__ amp_out,
-                                                               size_t plane, int P, int p0) {
+                                                               size_t plane, int q, int p0) {
     const size_t px = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (px >= plane) return;
     const int p = p0 + blockIdx.y;
@@ -661,7 +694,7 @@ __global__ void __launch_bounds__(256) phasenet_outputs_kernel(const float* __re
 #pragma unroll
     for (int c = 0; c < NB; ++c) {
         const size_t o = ((size_t)p * NB + c) * plane + px;
-        const float a1 = __ldg(amp + o), a2 = __ldg(amp + ((size_t)(P + p) * NB + c) * plane + px);
+        const float a1 = __ldg(amp + o), a2 = __ldg(amp + ((size_t)(q + p) * NB + c) * plane + px);
         const float beta = (v[NB + c] + 1.f) / 2.f;
         __stcs(phase_out + o, v[c] * 3.14159265358979323846f);
         __stcs(amp_out + o, beta * a2 + (1.f - beta) * a1);
@@ -716,31 +749,59 @@ extern "C" int fvfi_adacofnet_prep(const float* frame0, const float* frame2, flo
     return FVFI_OK;
 }
 
-extern "C" int fvfi_phasenet_assemble(const float* phase, const float* amp, const float* den, float* y, int y_pixel_stride, int P,
-                                      int p0, int pc, int nb, int H, int W, void* stream) {
-    FVFI_CHECK_ARG(phase && amp && den && y && P > 0 && p0 >= 0 && pc > 0 && p0 + pc <= P && pc <= 65535 && H > 0 && W > 0,
-                   "phasenet_assemble: bad argument");
-    FVFI_CHECK_ARG(nb == 4, "phasenet_assemble: nbands must be 4 (got %d)", nb);
-    FVFI_CHECK_ARG(y_pixel_stride >= 4 * nb, "phasenet_assemble: pixel stride smaller than 4*nbands");
+// Shared launches of the two glue kernels: the pair entry points pass N = 2P, q = P; the _offset ones take N and q from the caller.
+static int phasenet_assemble_launch(const char* name, const float* phase, const float* amp, const float* den, float* y,
+                                    int y_pixel_stride, int N, int P, int q, int p0, int pc, int nb, int H, int W, void* stream) {
+    FVFI_CHECK_ARG(phase && amp && den && y, "%s: null pointer", name);
+    FVFI_CHECK_ARG(P > 0 && p0 >= 0 && pc > 0 && p0 + pc <= P && pc <= 65535 && H > 0 && W > 0, "%s: bad argument", name);
+    FVFI_CHECK_ARG(q > 0 && (long long)p0 + pc - 1 + q < (long long)N, "%s: frame-2 plane offset q=%d out of range (N=%d, p0=%d, pc=%d)",
+                   name, q, N, p0, pc);
+    FVFI_CHECK_ARG(nb == 4, "%s: nbands must be 4 (got %d)", name, nb);
+    FVFI_CHECK_ARG(y_pixel_stride >= 4 * nb, "%s: pixel stride smaller than 4*nbands", name);
     const size_t plane = (size_t)H * W;
     dim3 grid((unsigned)((plane + 255) / 256), pc);
-    fvfi::phasenet_assemble_kernel<4><<<grid, 256, 0, (cudaStream_t)stream>>>(phase, amp, den, y, plane, y_pixel_stride, P, p0);
+    fvfi::phasenet_assemble_kernel<4><<<grid, 256, 0, (cudaStream_t)stream>>>(phase, amp, den, y, plane, y_pixel_stride, q, p0);
     FVFI_LAUNCH_CHECK();
     return FVFI_OK;
 }
 
-extern "C" int fvfi_phasenet_outputs(const float* pred, int pred_pixel_stride, const float* amp, float* phase_out, float* amp_out,
-                                     int P, int p0, int pc, int nb, int H, int W, void* stream) {
-    FVFI_CHECK_ARG(pred && amp && phase_out && amp_out && P > 0 && p0 >= 0 && pc > 0 && p0 + pc <= P && pc <= 65535 && H > 0 && W > 0,
-                   "phasenet_outputs: bad argument");
-    FVFI_CHECK_ARG(nb == 4, "phasenet_outputs: nbands must be 4 (got %d)", nb);
-    FVFI_CHECK_ARG(pred_pixel_stride >= 2 * nb, "phasenet_outputs: pixel stride smaller than 2*nbands");
+static int phasenet_outputs_launch(const char* name, const float* pred, int pred_pixel_stride, const float* amp, float* phase_out,
+                                   float* amp_out, int N, int P, int q, int p0, int pc, int nb, int H, int W, void* stream) {
+    FVFI_CHECK_ARG(pred && amp && phase_out && amp_out, "%s: null pointer", name);
+    FVFI_CHECK_ARG(P > 0 && p0 >= 0 && pc > 0 && p0 + pc <= P && pc <= 65535 && H > 0 && W > 0, "%s: bad argument", name);
+    FVFI_CHECK_ARG(q > 0 && (long long)p0 + pc - 1 + q < (long long)N, "%s: frame-2 plane offset q=%d out of range (N=%d, p0=%d, pc=%d)",
+                   name, q, N, p0, pc);
+    FVFI_CHECK_ARG(nb == 4, "%s: nbands must be 4 (got %d)", name, nb);
+    FVFI_CHECK_ARG(pred_pixel_stride >= 2 * nb, "%s: pixel stride smaller than 2*nbands", name);
     const size_t plane = (size_t)H * W;
     dim3 grid((unsigned)((plane + 255) / 256), pc);
-    fvfi::phasenet_outputs_kernel<4><<<grid, 256, 0, (cudaStream_t)stream>>>(pred, pred_pixel_stride, amp, phase_out, amp_out, plane, P,
+    fvfi::phasenet_outputs_kernel<4><<<grid, 256, 0, (cudaStream_t)stream>>>(pred, pred_pixel_stride, amp, phase_out, amp_out, plane, q,
                                                                              p0);
     FVFI_LAUNCH_CHECK();
     return FVFI_OK;
+}
+
+extern "C" int fvfi_phasenet_assemble(const float* phase, const float* amp, const float* den, float* y, int y_pixel_stride, int P,
+                                      int p0, int pc, int nb, int H, int W, void* stream) {
+    return phasenet_assemble_launch("phasenet_assemble", phase, amp, den, y, y_pixel_stride, 2 * P, P, P, p0, pc, nb, H, W, stream);
+}
+
+extern "C" int fvfi_phasenet_outputs(const float* pred, int pred_pixel_stride, const float* amp, float* phase_out, float* amp_out,
+                                     int P, int p0, int pc, int nb, int H, int W, void* stream) {
+    return phasenet_outputs_launch("phasenet_outputs", pred, pred_pixel_stride, amp, phase_out, amp_out, 2 * P, P, P, p0, pc, nb, H, W,
+                                   stream);
+}
+
+extern "C" int fvfi_phasenet_assemble_offset(const float* phase, const float* amp, const float* den, float* y, int y_pixel_stride,
+                                             int N, int P, int q, int p0, int pc, int nb, int H, int W, void* stream) {
+    return phasenet_assemble_launch("fvfi_phasenet_assemble_offset", phase, amp, den, y, y_pixel_stride, N, P, q, p0, pc, nb, H, W,
+                                    stream);
+}
+
+extern "C" int fvfi_phasenet_outputs_offset(const float* pred, int pred_pixel_stride, const float* amp, float* phase_out, float* amp_out,
+                                            int N, int P, int q, int p0, int pc, int nb, int H, int W, void* stream) {
+    return phasenet_outputs_launch("fvfi_phasenet_outputs_offset", pred, pred_pixel_stride, amp, phase_out, amp_out, N, P, q, p0, pc, nb,
+                                   H, W, stream);
 }
 
 // torch.cat of planar [B,c_s,H,W] tensors along the channels, written as ONE NHWC tensor (FusionNet's input,

@@ -61,6 +61,10 @@ _PROTOS = {
     "fvfi_upsample2_tapsum": (c_int, [c_fp, c_int, c_fp, c_fp, c_int, c_int, c_int, c_int, c_fp]),
     "fvfi_phasenet_assemble": (c_int, [c_fp, c_fp, c_fp, c_fp, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_fp]),
     "fvfi_phasenet_outputs": (c_int, [c_fp, c_int, c_fp, c_fp, c_fp, c_int, c_int, c_int, c_int, c_int, c_int, c_fp]),
+    "fvfi_phasenet_assemble_offset": (c_int, [c_fp, c_fp, c_fp, c_fp] + [c_int] * 9 + [c_fp]),
+    "fvfi_phasenet_outputs_offset": (c_int, [c_fp, c_int, c_fp, c_fp, c_fp] + [c_int] * 8 + [c_fp]),
+    "fvfi_rgb8_to_rgb_lab": (c_int, [c_fp, c_fp, c_fp, c_int, c_int, c_int, c_fp]),
+    "fvfi_fusion_blend_rgb8": (c_int, [c_fp, c_fp, c_fp, c_int, c_int, c_int, c_fp]),
     "fvfi_max_pool2_nhwc": (c_int, [c_fp, c_int, c_fp, c_int, c_int, c_int, c_int, c_int, c_fp]),
     "fvfi_adacofnet_prep": (c_int, [c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_int, c_int, c_int, c_int, c_int, c_fp, c_fp]),
     "fvfi_avg_pool2_nhwc": (c_int, [c_fp, c_int, c_fp, c_int, c_int, c_int, c_int, c_int, c_fp]),

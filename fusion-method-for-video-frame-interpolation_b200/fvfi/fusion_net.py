@@ -26,6 +26,21 @@ def fusion_blend(base, x):
     return out
 
 
+def fusion_blend_rgb8(base, x, out=None):
+    """The 8-bit form of ``fusion_blend``: planar [B,3,H,W] in, interleaved rgb24 [B,H,W,3] uint8 out,
+    rint(clamp(base + tanh(x), 0, 1) * 255) (ties to even); the fp32 frame is never stored (fvfi_fusion_blend_rgb8)."""
+    base = base.contiguous()
+    x = x.contiguous()
+    B, C, H, W = base.shape
+    assert C == 3 and x.shape == base.shape
+    if out is None:
+        out = torch.empty((B, H, W, 3), dtype=torch.uint8, device=base.device)
+    assert out.dtype == torch.uint8 and out.shape == (B, H, W, 3) and out.is_contiguous()
+    with torch.cuda.device(base.device):
+        _lib.check(_lib.lib().fvfi_fusion_blend_rgb8(base.data_ptr(), x.data_ptr(), out.data_ptr(), B, H, W, _lib.stream_ptr()))
+    return out
+
+
 class _FusionBlend(torch.autograd.Function):
     @staticmethod
     def forward(ctx, base, x):
@@ -90,6 +105,16 @@ class FusionNet(torch.nn.Module):
         ``Upsample(ReLU(x)) + skip`` and the final ``clamp(base + tanh)`` are the fused NHWC kernels; under autograd each of them is
         an autograd Function whose backward is a libfvfi kernel too (csrc/conv_bwd.cu) -- no ATen convolution / pooling /
         interpolation kernel runs in the training step of the trained network."""
+        x = self.residual(base, adacof, phase, other, maps)
+        anchor = phase if variant == 1 else base
+        if save:
+            self.residuals.append(torch.sum(torch.tanh(x.detach())).cpu().item())
+        return fusion_blend(anchor, x)
+
+    @tc.range_checked
+    def residual(self, base, adacof, phase, other, maps):
+        """The body of ``forward`` up to the pre-tanh residual x [B,3,H,W] (planar, contiguous): ``forward`` returns
+        ``fusion_blend(base, x)``; a caller that wants 8-bit frames ends with ``fusion_blend_rgb8(base, x)`` instead."""
         parts = [base, adacof, phase, other, maps]
         if not all(t.is_cuda for t in parts):
             raise NotImplementedError("fvfi FusionNet runs on CUDA tensors only (no CPU fallback)")
@@ -111,8 +136,4 @@ class FusionNet(torch.nn.Module):
             # Upsample(ReLU(x)) + skip as one pass (fvfi_resize_bilinear_nhwc_fused)
             x = tc.resize_bilinear(x, (x.shape[2] * 2, x.shape[3] * 2), False, relu_input=i > 0, add=s)
             x = tc.conv_module(layer, x, None)
-        x = x.contiguous()
-        anchor = phase if variant == 1 else base
-        if save:
-            self.residuals.append(torch.sum(torch.tanh(x.detach())).cpu().item())
-        return fusion_blend(anchor, x)
+        return x.contiguous()

@@ -166,13 +166,15 @@ class PhaseNet(nn.Module):
         return low_level, phases, amplitudes
 
     @tc.range_checked
-    def forward_fused(self, vals, amp_max, m=None):
+    def forward_fused(self, vals, amp_max, m=None, frame2=None):
         """Fused inference form of  separate_vals -> get_concat_layers_inf -> normalize_vals -> forward -> reverse_normalize
         (src/train/utils.py:47-127, phase_net.py:42-177) for two input frames.
 
-        ``vals``: the RAW decomposition (``Pyramid.filter``) of ``cat(frame-1 planes, frame-2 planes)`` (N = 2*P planes, lists finest
-        first); ``amp_max`` [L, N]: the per-level per-plane amplitude maxima from the decomposition's epilogue
-        (``Pyramid.last_amp_max``).  Returns the DecompValues ``Pyramid.inv_filter`` consumes (P planes).  The value channels of
+        ``vals``: the RAW decomposition (``Pyramid.filter``) of N planes, lists finest first, in which frame 2 of pair-plane p is
+        plane p + q, q = ``frame2``: the default N // 2 is ``cat(frame-1 planes, frame-2 planes)`` (N = 2*P); a clip of T'
+        consecutive frames decomposed once is q = 3 (pair t = frames t, t + 1), P = N - q.  ``amp_max`` [L, N]: the per-level
+        per-plane amplitude maxima from the decomposition's epilogue (``Pyramid.last_amp_max``).  Returns the DecompValues
+        ``Pyramid.inv_filter`` consumes (P planes).  The value channels of
         every level's concat are written by ONE kernel straight from the decomposition (fvfi_phasenet_assemble) and the amplitude
         blend + de-normalisation by another (fvfi_phasenet_outputs): the regrouped / normalised / re-scaled copies of the whole
         pyramid that the step-by-step form materialises (~80 GB per 8 frame pairs at 1080p) never exist."""
@@ -182,12 +184,14 @@ class PhaseNet(nn.Module):
         if m is None:
             m = self.pyr.height - 2
         N = vals.low_level.shape[0]
-        P = N // 2
+        q = N // 2 if frame2 is None else int(frame2)
+        P = N - q
+        assert 0 < q < N, (q, N)
         dev = vals.low_level.device
-        low = torch.cat((vals.low_level[:P], vals.low_level[P:]), 1)                       # [P,2,hL,wL] (a few hundred values)
+        low = torch.cat((vals.low_level[:P], vals.low_level[q:q + P]), 1)                  # [P,2,hL,wL] (a few hundred values)
         self.max_low_level = low.reshape(P, -1).max(1)[0] + self.eps                       # max, not max|.| (phase_net.py:70)
         low = low / self.max_low_level.view(-1, 1, 1, 1)
-        den = (torch.maximum(amp_max[:, :P], amp_max[:, P:]) + self.eps).contiguous()      # [L,P]: max over both frames' bands + eps
+        den = (torch.maximum(amp_max[:, :P], amp_max[:, q:q + P]) + self.eps).contiguous() # [L,P]: max over both frames' bands + eps
         self.max_amplitudes = [den[L - 1 - i] for i in range(m)]                           # coarsest first, as normalize_vals keeps them
         new = lambda *sh: torch.empty(sh, dtype=torch.float32, device=dev)
         phase_out = [new(P * nb, 1, *vals.phase[l].shape[2:]) if l >= L - m else 0 for l in range(L)]
@@ -216,8 +220,8 @@ class PhaseNet(nn.Module):
                     if cd != 2 * cv + cp:
                         direct.zero_()                                                     # padding channels must be finite
                     with torch.cuda.device(dev):
-                        _lib.check(lib.fvfi_phasenet_assemble(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(), direct.data_ptr(),
-                                                              direct.stride(3), P, p0, pc, nb, h, w, _lib.stream_ptr()))
+                        _lib.check(lib.fvfi_phasenet_assemble_offset(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(), direct.data_ptr(),
+                                                                     direct.stride(3), N, P, q, p0, pc, nb, h, w, _lib.stream_ptr()))
                     tc.resize_bilinear(prediction, (h, w), False, out=direct, out_channel_offset=2 * cv)
                     feature, prediction = self.layers[i].forward_resampled(feature, direct, (h, w))
                     del direct
@@ -226,16 +230,16 @@ class PhaseNet(nn.Module):
                                          memory_format=torch.channels_last)
                     tc.resize_bilinear(feature, (h, w), False, out=concat, out_channel_offset=0)
                     with torch.cuda.device(dev):
-                        _lib.check(lib.fvfi_phasenet_assemble(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(),
-                                                              concat.data_ptr() + 4 * cf, concat.stride(3), P, p0, pc, nb, h, w,
-                                                              _lib.stream_ptr()))
+                        _lib.check(lib.fvfi_phasenet_assemble_offset(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(),
+                                                                     concat.data_ptr() + 4 * cf, concat.stride(3), N, P, q, p0, pc, nb,
+                                                                     h, w, _lib.stream_ptr()))
                     tc.resize_bilinear(prediction, (h, w), False, out=concat, out_channel_offset=cf + 2 * cv)
                     feature, prediction = self.layers[i](concat)
                     del concat
                 pr = tc.to_nhwc(prediction)
                 with torch.cuda.device(dev):
-                    _lib.check(lib.fvfi_phasenet_outputs(pr.data_ptr(), pr.stride(3), am.data_ptr(), phase_out[l].data_ptr(),
-                                                         amp_out[l].data_ptr(), P, p0, pc, nb, h, w, _lib.stream_ptr()))
+                    _lib.check(lib.fvfi_phasenet_outputs_offset(pr.data_ptr(), pr.stride(3), am.data_ptr(), phase_out[l].data_ptr(),
+                                                                amp_out[l].data_ptr(), N, P, q, p0, pc, nb, h, w, _lib.stream_ptr()))
         low_level = (lows[0] if len(lows) == 1 else torch.cat(lows, 0)) * self.max_low_level.view(-1, 1, 1, 1)
         H, W = int(vals.phase[0].shape[2]), int(vals.phase[0].shape[3])
         high_level = torch.zeros((1,), dtype=torch.float32, device=dev).expand(P, 1, H, W)  # zeros (phase_net.py:127-128), no storage

@@ -17,7 +17,7 @@ import torch
 from . import conv as tc
 from . import filters, transform, utils
 from .adacofnet import AdaCoFNet
-from .fusion_net import FusionNet
+from .fusion_net import FusionNet, fusion_blend_rgb8
 from .phase_net import PhaseNet
 from .pyramid import Pyramid
 
@@ -135,9 +135,18 @@ class FusionPipeline(torch.nn.Module):
         under no_grad, src/fusion_net/trainer.py:65-213)."""
         B, _, H, W = rgb1.shape
         assert (H, W) == (self.H, self.W) and rgb2.shape == rgb1.shape
-        pyr, r_shape = self.pyr, (B, 3, H, W)
         self._tick('start')
         lab1, lab2 = transform.rgb2lab(rgb1), transform.rgb2lab(rgb2)                           # :148-149
+        planes = torch.cat((lab1.reshape(-1, H, W), lab2.reshape(-1, H, W)), 0)
+        return self._fusion_inputs(rgb1, rgb2, lab1, lab2, planes, 3 * B)
+
+    def _fusion_inputs(self, rgb1, rgb2, lab1, lab2, planes, q):
+        """The pair-dependent body of ``fusion_inputs``: frames rgb1 / rgb2 [B,3,H,W], their Lab lab1 / lab2 and the Lab planes
+        [N,H,W] the PhaseNet branch decomposes, in which frame 2 of pair-plane p is plane p + q.  Pairs: planes = cat(lab1, lab2),
+        q = 3B.  A clip of B + 1 frames: planes = Lab of the B + 1 frames (each decomposed once), q = 3, and rgb1 / rgb2 / lab1 /
+        lab2 are the views frames[:-1] / frames[1:]."""
+        B, _, H, W = rgb1.shape
+        pyr, r_shape = self.pyr, (B, 3, H, W)
         fork = self.concurrent_small and H * W <= 512 * 512 and self.timing is None
         if fork:
             main = torch.cuda.current_stream(rgb1.device)
@@ -153,14 +162,14 @@ class FusionPipeline(torch.nn.Module):
             flow_var_map = flow_var_map.squeeze(1)
         self._tick('lab+adacofnet#1')
         # PhaseNet branch (:168-192)
-        vals = self._filter("phasenet", torch.cat((lab1.reshape(-1, H, W), lab2.reshape(-1, H, W)), 0), want_high=False)
+        vals = self._filter("phasenet", planes, want_high=False)
         self._tick('pyr.filter(12 planes/frame)')
         if self.fused_phase_glue:
             # separate_vals / get_concat_layers_inf / normalize_vals / forward / reverse_normalize with the regrouping and the
             # (de)normalisation fused into the concat assembly and the output kernel (PhaseNet.forward_fused)
-            vals_pred = self.phase_net.forward_fused(vals, pyr.last_amp_max)
+            vals_pred = self.phase_net.forward_fused(vals, pyr.last_amp_max, frame2=q)
         else:
-            vals_in = self.phase_net.normalize_vals(utils.get_concat_layers_inf(pyr, utils.separate_vals(vals, 2)))
+            vals_in = self.phase_net.normalize_vals(utils.get_concat_layers_inf(pyr, utils.pair_vals(vals, q, pyr.nbands)))
             vals_pred = self.phase_net(vals_in)
             del vals_in
         del vals
@@ -268,44 +277,137 @@ class FusionPipeline(torch.nn.Module):
                 self.stages["phase%d" % l], self.stages["amp%d" % l] = p, a
         return phase_pred
 
+    def _check_clip(self, frames):
+        """Validates a clip for interpolate_sequence; returns True for 8-bit [T,H,W,3], False for fp32 [T,3,H,W]."""
+        if not torch.is_tensor(frames) or frames.dim() != 4:
+            raise ValueError("a clip is a 4-d tensor: float32 [T,3,H,W] or uint8 [T,H,W,3]")
+        if frames.dtype == torch.uint8:
+            shape, want = tuple(frames.shape[1:]), (self.H, self.W, 3)
+        elif frames.dtype == torch.float32:
+            shape, want = tuple(frames.shape[1:]), (3, self.H, self.W)
+        else:
+            raise ValueError("clip dtype must be torch.float32 ([T,3,H,W] in [0,1]) or torch.uint8 ([T,H,W,3]), got %s" % frames.dtype)
+        if shape != want:
+            raise ValueError("%s clip frames must be %s for this %dx%d pipeline, got %s (wrong frame size or layout)"
+                             % (frames.dtype, list(want), self.W, self.H, list(shape)))
+        if frames.shape[0] < 2:
+            raise ValueError("a clip needs at least 2 frames, got %d" % frames.shape[0])
+        return frames.dtype == torch.uint8
+
+    def _clip_window(self, frames, out=None):
+        """Interpolates the B pairs of a window of B + 1 consecutive frames (device tensors in interpolate_sequence's formats):
+        Lab and the pyramid decomposition run once per frame, the pairs read them as views (clip layout, q = 3).  Writes the B new
+        frames into ``out`` (allocated if None) in the input's dtype and layout."""
+        H, W = self.H, self.W
+        self._tick('start')
+        if frames.dtype == torch.uint8:
+            rgb, lab = transform.rgb8_to_rgb_lab(frames)
+        else:
+            rgb = frames.contiguous()
+            lab = transform.rgb2lab(rgb)
+        base, ada_pred, phase_pred, other, maps = self._fusion_inputs(rgb[:-1], rgb[1:], lab[:-1], lab[1:], lab.reshape(-1, H, W), 3)
+        if frames.dtype == torch.uint8:
+            x = self.fusion_net.residual(base, ada_pred, phase_pred, other, maps)
+            out = fusion_blend_rgb8(base, x, out)
+        else:
+            final = self.fusion_net(base, ada_pred, phase_pred, other, maps, variant=0)
+            out = final if out is None else out.copy_(final)
+        self._tick('fusion_net')
+        return out
+
+    @torch.no_grad()
+    @tc.range_checked
+    def interpolate_sequence(self, frames):
+        """The T - 1 in-between frames of a clip on the device: fp32 [T,3,H,W] in [0,1] -> fp32 [T-1,3,H,W], or uint8 [T,H,W,3]
+        (rgb24) -> uint8 [T-1,H,W,3] (8-bit in and out: no fp32 frame is stored at either end).  Frame t of the result lies
+        between input frames t and t + 1.  Works in windows of ``max_batch`` pairs; a window of B pairs converts and decomposes
+        its B + 1 frames once (the pair form ``pipe(frames[:-1], frames[1:])`` does every interior frame twice); the frame
+        between two windows is done again in the next one.  ValueError for fewer than 2 frames, a wrong frame size, dtype or
+        layout."""
+        u8 = self._check_clip(frames)
+        if not frames.is_cuda:
+            raise ValueError("interpolate_sequence takes device tensors (interpolate_video_host takes host frames)")
+        T, mb = frames.shape[0], self.max_batch
+        out = torch.empty((T - 1,) + tuple(frames.shape[1:]), dtype=torch.uint8 if u8 else torch.float32, device=frames.device)
+        for a in range(0, T - 1, mb):
+            b = min(mb, T - 1 - a)
+            self._clip_window(frames[a:a + b + 1], out[a:a + b])
+        return out
+
+    def interpolate_video_host(self, frames_host, out_host=None):
+        """Clip on HOST (pinned) memory: uint8 [T,H,W,3] rgb24 -> uint8 [2T-1,H,W,3], the input frames at even indices and the
+        interpolated ones at odd indices (twice the frame rate).  Windows of ``max_batch`` pairs go up as 8-bit frames and come
+        back as 8-bit frames on the two copy streams of interpolate_host, overlapped with the compute of the neighbouring
+        windows; the input frames are copied into the even slots on the host meanwhile."""
+        if not torch.is_tensor(frames_host) or frames_host.is_cuda or frames_host.dtype != torch.uint8:
+            raise ValueError("interpolate_video_host takes a host uint8 [T,H,W,3] tensor (pinned for overlapped copies)")
+        self._check_clip(frames_host)
+        frames_host = frames_host.contiguous()
+        T, H, W = frames_host.shape[0], self.H, self.W
+        if out_host is None:
+            out_host = torch.empty((2 * T - 1, H, W, 3), dtype=torch.uint8).pin_memory()
+        if tuple(out_host.shape) != (2 * T - 1, H, W, 3) or out_host.dtype != torch.uint8 or out_host.is_cuda:
+            raise ValueError("out_host must be a host uint8 [%d,%d,%d,3] tensor" % (2 * T - 1, H, W))
+        mb = self.max_batch
+        starts = list(range(0, T - 1, mb))
+        uploads = [(frames_host[a:a + min(mb, T - 1 - a) + 1],) for a in starts]
+
+        def download(k, out):                  # per-frame contiguous views of the odd slots
+            for i in range(out.shape[0]):
+                out_host[2 * (starts[k] + i) + 1].copy_(out[i], non_blocking=True)
+
+        def host_work():
+            out_host[0::2].copy_(frames_host)
+        self._run_windows(uploads, self._clip_window, download, host_work)
+        return out_host
+
     def interpolate_host(self, rgb1_host, rgb2_host, out_host=None):
         """End-to-end call on HOST (pinned) tensors [B,3,H,W]: host -> device copies of the frames, the pipeline, device -> host
         copy of the result, all inside the call.  The batch is processed in sub-batches of ``max_batch`` pairs; the copies run
         on two side streams, so sub-batch k+1's frames arrive and sub-batch k-1's result leaves while sub-batch k computes."""
-        B = rgb1_host.shape[0]
+        B, mb = rgb1_host.shape[0], self.max_batch
         if out_host is None:
             out_host = torch.empty((B, 3, self.H, self.W), dtype=torch.float32).pin_memory()
-        if self._copy_streams is None:
-            self._copy_streams = (torch.cuda.Stream(self.device), torch.cuda.Stream(self.device))
-        self._interp_chunks(rgb1_host, rgb2_host, out_host)
+        starts = list(range(0, B, mb))
+        uploads = [(rgb1_host[a:a + mb], rgb2_host[a:a + mb]) for a in starts]
+
+        def download(k, out):
+            out_host[starts[k]:starts[k] + out.shape[0]].copy_(out, non_blocking=True)
+        self._run_windows(uploads, self.forward, download)
         return out_host
 
     @torch.no_grad()
-    @tc.range_checked       # ONE range check (stream sync) for the whole call; the sub-batch forwards below are nested in it
-    def _interp_chunks(self, h1, h2, out_host):
+    @tc.range_checked       # ONE range check (stream sync) for the whole call; the per-window calls below are nested in it
+    def _run_windows(self, uploads, run, download, host_work=None):
+        """Stream choreography of the host-buffer entry points: ``uploads`` [k] is the tuple of host tensors of window k; their
+        host -> device copies are all queued at once on the input stream (in order), window k's ``run(*device_tensors)`` waits for
+        its own copies only, and ``download(k, result)`` issues its device -> host copies on the output stream after the window's
+        compute.  ``host_work()`` (optional) runs on the host while the device works; the call returns with every result on the
+        host."""
+        if self._copy_streams is None:
+            self._copy_streams = (torch.cuda.Stream(self.device), torch.cuda.Stream(self.device))
         compute = torch.cuda.current_stream(self.device)
         s_in, s_out = self._copy_streams
-        B, mb = h1.shape[0], self.max_batch
         s_in.wait_stream(compute)                      # the caller's earlier work on these buffers is ordered before the copies
         staged = []
-        for a in range(0, B, mb):                      # all uploads are queued at once; they run in order on the input stream
+        for hs in uploads:                             # all uploads are queued at once; they run in order on the input stream
             with torch.cuda.stream(s_in):
-                d1 = h1[a:a + mb].to(self.device, non_blocking=True)
-                d2 = h2[a:a + mb].to(self.device, non_blocking=True)
+                ds = [h.to(self.device, non_blocking=True) for h in hs]
                 ev = torch.cuda.Event()
                 ev.record(s_in)
-            staged.append((a, d1, d2, ev))
-        for a, d1, d2, ev in staged:
+            staged.append((ds, ev))
+        for k, (ds, ev) in enumerate(staged):
             compute.wait_event(ev)
-            d1.record_stream(compute)
-            d2.record_stream(compute)
-            out = self.forward(d1, d2)
+            for d in ds:
+                d.record_stream(compute)
+            out = run(*ds)
             done = torch.cuda.Event()
             done.record(compute)
             with torch.cuda.stream(s_out):
                 s_out.wait_event(done)
-                out_host[a:a + out.shape[0]].copy_(out, non_blocking=True)
+                download(k, out)
             out.record_stream(s_out)
+        if host_work is not None:
+            host_work()
         compute.wait_stream(s_out)                     # the call returns with the result on the host
         compute.synchronize()
-        return out_host

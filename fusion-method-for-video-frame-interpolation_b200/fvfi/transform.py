@@ -36,6 +36,21 @@ def lab2rgb(img, light=100, ab_mul=255, ab_max=128):
     return _run("fvfi_lab2rgb", img)
 
 
+def rgb8_to_rgb_lab(frames8):
+    """Decoder frames [T,H,W,3] uint8 (interleaved rgb24) -> (rgb, lab): planar fp32 [T,3,H,W] RGB (the correctly rounded k / 255)
+    and scaled Lab, in one kernel (fvfi_rgb8_to_rgb_lab); ``lab`` equals ``rgb2lab(rgb)`` bit for bit."""
+    if not frames8.is_cuda:
+        raise NotImplementedError("fvfi colour transforms run on CUDA tensors only")
+    assert frames8.dtype == torch.uint8 and frames8.dim() == 4 and frames8.shape[3] == 3
+    x = frames8.contiguous()
+    T, H, W, _ = x.shape
+    rgb = torch.empty((T, 3, H, W), dtype=torch.float32, device=x.device)
+    lab = torch.empty_like(rgb)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().fvfi_rgb8_to_rgb_lab(x.data_ptr(), rgb.data_ptr(), lab.data_ptr(), T, H, W, _lib.stream_ptr()))
+    return rgb, lab
+
+
 def lab2rgb_single(img, light=100, ab_mul=255, ab_max=128):
     """[3,H,W] (transform.py:40-49)."""
     return lab2rgb(img.unsqueeze(0), light, ab_mul, ab_max)[0]

@@ -101,6 +101,9 @@ int fvfi_adacofnet_warp_blend_rows(const float* in1, const float* in2, const flo
 
 /* FusionNet's last step (src/fusion_net/fusion_net.py:67-77): out = clamp(base + tanh(x), 0, 1). */
 int fvfi_fusion_blend(const float* base, const float* x_pre_tanh, float* out, size_t n, void* stream);
+/* The same blend for 8-bit output: base / x_pre_tanh [B,3,H,W] planar -> out [B,H,W,3] uint8 interleaved (rgb24),
+ * out = rint(clamp(base + tanh(x), 0, 1) * 255) with ties to even.  The fp32 frame is never written. */
+int fvfi_fusion_blend_rgb8(const float* base, const float* x_pre_tanh, uint8_t* out, int B, int H, int W, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Per-pixel stages the reference runs on the host CPU (SURVEY.md 8(f) f1/f2), device-resident here.
@@ -108,6 +111,9 @@ int fvfi_fusion_blend(const float* base, const float* x_pre_tanh, float* out, si
  * then L/100 and (a,b+128)/255). */
 int fvfi_rgb2lab(const float* rgb, float* lab, int B, int H, int W, void* stream);
 int fvfi_lab2rgb(const float* lab, float* rgb, int B, int H, int W, void* stream);
+/* Decoder frames rgb8 [T,H,W,3] uint8 interleaved (ffmpeg -pix_fmt rgb24) -> rgb [T,3,H,W] planar fp32 (the correctly rounded
+ * k / 255) and lab [T,3,H,W] planar scaled Lab, in one pass; lab is bit-identical to fvfi_rgb2lab of rgb. */
+int fvfi_rgb8_to_rgb_lab(const uint8_t* rgb8, float* rgb, float* lab, int T, int H, int W, void* stream);
 /* scipy.ndimage.gaussian_filter(x, sigma) on N maps [N,H,W] (truncate 4, mode 'reflect';
  * src/fusion_net/interpolate_twoframe.py:212-213).  tmp: scratch of the same size. */
 int fvfi_gaussian_filter(const float* in, float* out, float* tmp, int N, int H, int W, float sigma, void* stream);
@@ -243,6 +249,13 @@ int fvfi_phasenet_assemble(const float* phase, const float* amp, const float* de
                            int p0, int pc, int nb, int H, int W, void* stream);
 int fvfi_phasenet_outputs(const float* pred, int pred_pixel_stride, const float* amp, float* phase_out, float* amp_out,
                           int P, int p0, int pc, int nb, int H, int W, void* stream);
+/* The same two steps for any plane layout: phase / amp hold N planes and frame 2 of pair-plane p is plane p + q (the two entry
+ * points above are q = P, N = 2P).  A clip of T' consecutive frames decomposed once is q = 3, P = N - 3: pair t reads frames t and
+ * t + 1.  FVFI_EINVAL if p0 + pc - 1 + q >= N. */
+int fvfi_phasenet_assemble_offset(const float* phase, const float* amp, const float* den, float* y, int y_pixel_stride, int N, int P,
+                                  int q, int p0, int pc, int nb, int H, int W, void* stream);
+int fvfi_phasenet_outputs_offset(const float* pred, int pred_pixel_stride, const float* amp, float* phase_out, float* amp_out, int N,
+                                 int P, int q, int p0, int pc, int nb, int H, int W, void* stream);
 
 /* Bilinear resize of NHWC tensors (torch.nn.Upsample / F.interpolate 'bilinear' semantics, both align_corners
  * modes; src/fusion_net/fusion_adacofnet.py:31, src/fusion_net/fusion_net.py:41, src/phase_net/phase_net.py:138-139).
