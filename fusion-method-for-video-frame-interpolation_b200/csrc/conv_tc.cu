@@ -1002,11 +1002,7 @@ static int conv_geometry(ConvArgs& a, int prec, size_t* smem_bytes) {
         // consecutive loader lanes store) then start 32 bytes apart modulo the 128-byte bank row, and a quarter-warp's 128-bit
         // stores (two pixels x four K chunks) cover all 32 banks once (ncu on 32->32 @1088x1920: the unpadded stride put K chunks
         // 0/2 and 1/3 on the same banks -- 8 instead of 4 wavefronts per STS.128, 20 M of the layer's 150 M LSU wavefronts)
-#ifdef FVFI_CONV_NO_KCS_PAD
-        a.KCS = a.NPIX;
-#else
         a.KCS = a.NPIX + ((2 - a.NPIX) & 7);
-#endif
         a.a_stage_bytes = (unsigned)a.KCS * CV_KCHUNKS * 16u * 2u;    // hi + lo
         if (a.NPIX * CV_KCHUNKS > CV_LOADERS * CV_UMAX) continue;          // the loaders keep a whole K chunk in registers (UMAX)
         const size_t misc = 512 + (size_t)a.NPIX * 4 + 1024 + 16 + (a.up ? (size_t)a.NPIX * 16 : 0);

@@ -10,12 +10,14 @@
 //     decimation-in-frequency network whose digit-reversed output order is free (a column pass writes 64-byte row
 //     segments, their order does not matter) -- half the shared memory, twice the resident CTAs.
 //   * lengths n = r * p with ONE prime factor p > 19 whose p - 1 is smooth (97, 191, 241, 61, 43, 31, 23 ... -- every such
-//     length of the 1080p / 4K pyramids): Cooley-Tukey split into r interleaved length-p DFTs (ordinary in-place DIF stages
-//     for the radices of r), each done by RADER's algorithm: a length-p DFT is y0 plus a cyclic convolution of length p - 1
-//     of the inputs taken in the order g^q (g a primitive root of p) with the constant sequence W_p^(g^-q).  The convolution
-//     runs on the same stage code as everything else: one permuting copy into the second buffer, in-place DIF of the
-//     (p-1)-point sub-sequences, multiply by the precomputed spectrum (stored in DIF order, DC bin carries y0), in-place
-//     DIT back -- no zero padding, all passes over n points instead of Bluestein's M >= 2n - 1.
+//     length of the 1080p / 4K pyramids): decimation in time into r interleaved length-p DFTs, each done by RADER's
+//     algorithm: a length-p DFT is y0 plus a cyclic convolution of length p - 1 of the inputs taken in the order g^q
+//     (g a primitive root of p) with the constant sequence W_p^(g^-q).  fft_put scatters every input straight to its
+//     residue block and generator-order slot (pos_in), so the whole transform runs in place in ONE buffer of n slots:
+//     in-place DIF of the (p-1)-point sub-sequences, multiply by the precomputed spectrum (stored in DIF order, DC bin
+//     carries y0), in-place DIT back, then the in-place DIT radix stages of r across the blocks (their twiddle index goes
+//     through `perm`, the blocks being in generator order) -- no zero padding and no copy pass, all passes over n points
+//     instead of Bluestein's M >= 2n - 1.
 //   * other lengths: Bluestein (chirp-z) on a smooth length M >= 2n-1 chosen by the plan: chirp, in-place DIF,
 //     multiply by the precomputed spectrum of the chirp filter (stored in DIF order, pre-scaled by 1/M), in-place
 //     DIT (digit-reversed in, natural out), chirp.  No permutation pass anywhere, and no extra pass either: the
@@ -43,14 +45,12 @@ constexpr int FFT_MAX_STAGES = 8;
 
 struct FftPlan {
     int n;                       // logical transform length
-    int M;                       // machine length: n (direct, Rader) or the Bluestein convolution length
-    int alloc;                   // slots per sequence the caller provides: M, or 2n for Rader in the column layout (two halves)
+    int M;                       // machine length and slots per sequence: n (direct, Rader) or the Bluestein convolution length
     int nfac;
     int bluestein;
-    int rader;                   // n = rr * rp, stages [0, nouter) work on length n, stages [nouter, nfac) are the sub-FFT of length rq.
-                                 // 1: decimation in frequency (outer DIF stages, permuting copy into a second buffer, Rader);
-                                 // 2: decimation in time (inputs scattered by pos_in on the way in, Rader in place, outer DIT stages
-                                 //    whose twiddle index goes through `perm`): no copy pass, ONE buffer of n slots
+    int rader;                   // 1: n = rr * rp by decimation in time (inputs scattered by pos_in on the way in, Rader in place,
+                                 // outer DIT stages whose twiddle index goes through `perm`); stages [0, nouter) work on length n,
+                                 // stages [nouter, nfac) are the sub-FFT of length rq
     int rr, rp, rq, nouter;      // rq = rp - 1
     int pad;                     // sequence-major layout: 1 = skew i + (i >> 4) (smallest butterfly stride is even)
     int fac[FFT_MAX_STAGES];     // radices in network order (product = M; Rader: product = rr * rq)
@@ -58,15 +58,13 @@ struct FftPlan {
     unsigned mag_sub[FFT_MAX_STAGES];    // ceil(2^32 / sub)
     unsigned mag_items[FFT_MAX_STAGES];  // ceil(2^32 / (M / fac));  Rader sub stages: ceil(2^32 / (rq / fac))
     unsigned mag_ritems[FFT_MAX_STAGES]; // Rader sub stages: ceil(2^32 / (rr * rq / fac))
-    unsigned mag_rp;             // ceil(2^32 / rp)
     const float2* tw;            // W_M^t = exp(-2 pi i t / M), t < M
     const unsigned short* perm;  // direct DIF / Rader: natural index held at position p after the network (null: natural)
     const float2* chirp;         // Bluestein: exp(-i pi k^2 / n), k < n
     const float2* bhat;          // Bluestein: FFT_M(chirp filter) / M in DIF (digit-reversed) order;  Rader: FFT_rq(W_rp^(g^-t)) / rq, DIF order
     const float2* tw2;           // Rader: W_rq^t, t < rq
-    const unsigned short* pin;   // Rader: slot of input j inside its length-rp block (0 for j = 0, 1 + dlog_g(j) otherwise)
     const unsigned short* inv;   // Rader: position of natural index k in the result (sequence-major layout reads in natural order)
-    const unsigned short* pos_in; // Rader (decimation in time): position input i is written to
+    const unsigned short* pos_in; // Rader: position input i is written to
 };
 
 struct FftCtx { int tid, nthr; };
@@ -336,7 +334,7 @@ FVFI_HD void fft_stage_impl(const FftPlan& P, int s, const float2* in, float2* o
                 v[u] = LINEAR ? in[a0 + u * st] : in[fft_addr<COL>(b, base + u * m, ctshift, pitch, 1)];
             if (KIND == FFT_DIT && m > 1) {
                 // decimation-in-time Rader: the length-m blocks hold their spectrum in generator order; `perm` names the frequency
-                const int jf = (P.rader == 2) ? (int)ldg_(P.perm + j) : j;
+                const int jf = P.rader ? (int)ldg_(P.perm + j) : j;
                 twiddle_powers<R>(v, ldg_(tw + jf * (M / (R * m))));
             }
             dft(v, Radix<R>());
@@ -356,8 +354,8 @@ FVFI_HD void fft_stage_impl(const FftPlan& P, int s, const float2* in, float2* o
 
 // Rader sub-FFT stage: in-place DIF / DIT butterflies on the (p-1)-point sub-sequences that sit at offset 1 of every length-p
 // block of `buf` (rr blocks per sequence).  POST (last DIF stage): multiply by the convolution spectrum, fold y0 (slot 0 of the
-// block) into the DC bin, leave conj(X[0]) in slot 0, conjugate (the inverse transform is conj -> forward DIT -> conj, the last
-// conj being applied by fft_get).
+// block) into the DC bin, leave X[0] in slot 0, conjugate (the inverse transform is conj -> forward DIT -> conj, the last conj
+// being applied by the last DIT stage).
 template <int R, int KIND, bool COL>
 FVFI_HD void fft_stage_sub_impl(const FftPlan& P, int s, float2* buf, int batch, int ctshift, int pitch, const float2* post,
                                 FftCtx cx) {
@@ -394,33 +392,17 @@ FVFI_HD void fft_stage_sub_impl(const FftPlan& P, int s, float2* buf, int batch,
                 if (u == 0 && base == 0) {                    // DC bin of this block: X[0] = y0 + sum, and y0 rides on every output
                     const int a00 = fft_addr<COL>(b, blk * rp, ctshift, pitch, 0);
                     const float2 y0 = buf[a00];
-                    const float2 x0 = cadd(y0, v[0]);
-                    buf[a00] = (P.rader == 2) ? x0 : cconj(x0);   // DIF variant: fft_get conjugates every slot; DIT variant: final value
+                    buf[a00] = cadd(y0, v[0]);
                     w = cadd(w, y0);
                 }
                 v[u] = cconj(w);
             }
         }
-        // decimation-in-time variant: the last stage of the inverse sub-transform finishes the conj -> forward -> conj identity here
-        // (the outer radix stages that follow need the true block spectra)
-        const bool conj_out = KIND == FFT_DIT && P.rader == 2 && s == P.nouter;
+        // the last stage of the inverse sub-transform finishes the conj -> forward -> conj identity here (the outer radix stages
+        // that follow need the true block spectra)
+        const bool conj_out = KIND == FFT_DIT && s == P.nouter;
 #pragma unroll
         for (int u = 0; u < R; ++u) buf[a0 + u * st] = conj_out ? cconj(v[u]) : v[u];
-    }
-}
-
-// Rader: copy the natural-order blocks of `src` into `dst` in generator order (slot pin[j] of the same block).
-template <bool COL>
-FVFI_HD void fft_rader_permute(const FftPlan& P, const float2* src, float2* dst, int batch, int ctshift, int pitch, FftCtx cx) {
-    const int n = P.n, rp = P.rp, total = batch * n;
-    const unsigned mag_rp = P.mag_rp;
-    const unsigned short* pin = P.pin;
-    for (int q = cx.tid; q < total; q += cx.nthr) {
-        int b, i;
-        if (COL) { i = q >> ctshift; b = q & ((1 << ctshift) - 1); } else { b = q / n; i = q - b * n; }
-        const int blk = (int)fast_div((unsigned)i, (unsigned)rp, mag_rp);
-        const int j = i - blk * rp;
-        dst[fft_addr<COL>(b, blk * rp + (int)ldg_(pin + j), ctshift, pitch, 0)] = src[fft_addr<COL>(b, i, ctshift, pitch, 0)];
     }
 }
 
@@ -494,7 +476,7 @@ struct FftIO {
 FVFI_HD FftIO fft_io(const FftPlan& P) { return FftIO{P.bluestein, P.pad, P.rader, P.chirp, P.inv, P.pos_in}; }
 
 // Pitch (floats2 per sequence) of the sequence-major layout for this plan.
-FVFI_HD int fft_pitch(const FftPlan& P) { return fft_row_pitch(P.alloc, P.pad); }
+FVFI_HD int fft_pitch(const FftPlan& P) { return fft_row_pitch(P.M, P.pad); }
 
 // Callers WRITE their input through fft_put (Bluestein: the chirp is applied on the way in) ...
 template <bool COL>
@@ -509,8 +491,7 @@ template <bool COL>
 FVFI_HD float2 fft_get(const FftIO& io, const FftResult& R, int b, int pos, int ctshift, int pitch) {
     if (io.rader) {      // result sits in generator order: the column layout walks positions (R.perm names them), rows look them up
         const int p2 = COL ? pos : (int)ldg_(io.inv + pos);
-        const float2 v = R.buf[fft_addr<COL>(b, p2, ctshift, pitch, 0)];
-        return io.rader == 2 ? v : cconj(v);              // decimation in time has already conjugated (before its outer stages)
+        return R.buf[fft_addr<COL>(b, p2, ctshift, pitch, 0)];
     }
     const float2 v = R.buf[fft_addr<COL>(b, pos, ctshift, pitch, io.pad)];
     return io.bluestein ? cmul(cconj(v), ldg_(io.chirp + pos)) : v;
@@ -527,9 +508,9 @@ template <bool COL>
 FVFI_HD FftResult fft_forward(const FftPlan& P, float2* a, float2* b, int batch, int ctshift, int pitch, bool inplace,
                               FftCtx cx, int src_plain = 0) {
     const int M = P.M, n = P.n, pad = P.pad;
-    if (P.rader == 2) {
-        // decimation in time: fft_put has scattered the inputs into residue blocks in generator order; Rader on every block in
-        // place, then the radix stages of r across the blocks (twiddle index through `perm`: the blocks are in generator order)
+    if (P.rader) {
+        // fft_put has scattered the inputs into residue blocks in generator order; Rader on every block in place, then the
+        // radix stages of r across the blocks (twiddle index through `perm`: the blocks are in generator order)
         for (int s = P.nouter; s < P.nfac; ++s) {
             fft_run_stage_sub<FFT_DIF, COL>(P, s, a, batch, ctshift, pitch, s == P.nfac - 1 ? P.bhat : nullptr, cx);
             fft_sync();
@@ -543,24 +524,6 @@ FVFI_HD FftResult fft_forward(const FftPlan& P, float2* a, float2* b, int batch,
             fft_sync();
         }
         return FftResult{a, P.perm};
-    }
-    if (P.rader) {
-        for (int s = 0; s < P.nouter; ++s) {                 // Cooley-Tukey stages for the smooth part r of n = r * p
-            fft_run_stage<FFT_DIF, COL>(P, s, a, a, batch, ctshift, pitch, nullptr, cx);
-            fft_sync();
-        }
-        float2* w = COL ? a + ((size_t)n << ctshift) : b;    // second half (column tile) / second buffer (rows)
-        fft_rader_permute<COL>(P, a, w, batch, ctshift, pitch, cx);
-        fft_sync();
-        for (int s = P.nouter; s < P.nfac; ++s) {
-            fft_run_stage_sub<FFT_DIF, COL>(P, s, w, batch, ctshift, pitch, s == P.nfac - 1 ? P.bhat : nullptr, cx);
-            fft_sync();
-        }
-        for (int s = P.nfac - 1; s >= P.nouter; --s) {
-            fft_run_stage_sub<FFT_DIT, COL>(P, s, w, batch, ctshift, pitch, nullptr, cx);
-            fft_sync();
-        }
-        return FftResult{w, P.perm};
     }
     if (P.bluestein) {
         const int tail = M - n;                              // zero padding of the convolution

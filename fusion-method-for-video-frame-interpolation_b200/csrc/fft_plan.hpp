@@ -16,13 +16,6 @@ struct HostFftPlan {
     std::vector<unsigned short> perm, pin, inv, pos_in;
 };
 
-// Test / A-B switch: 0 makes every non-smooth length use Bluestein (round-1 behaviour); 1 = Rader, decimation in frequency
-// (permuting copy, two buffers); 2 = Rader, decimation in time (default: no copy pass, one buffer).
-inline int& fft_rader_enabled() {
-    static int on = 2;
-    return on;
-}
-
 // Split n into the radices the engine implements; false if n has a prime factor > 19.
 inline bool fft_radices(int n, std::vector<int>& out) {
     out.clear();
@@ -121,8 +114,8 @@ inline bool fft_rader_split(int n, int* r_out, int* p_out) {
     return true;
 }
 
-// Rader plan (see fft_engine.cuh): outer DIF stages for r, sub-FFT stages for q = p - 1, generator-order tables.
-inline bool fft_make_rader_plan(int n, int r, int pr, bool column_layout, HostFftPlan& H, int variant = 1) {
+// Rader plan (see fft_engine.cuh): outer DIT stages for r, sub-FFT stages for q = p - 1, generator-order tables.
+inline bool fft_make_rader_plan(int n, int r, int pr, HostFftPlan& H) {
     FftPlan& p = H.p;
     const int q = pr - 1;
     std::vector<int> rad_r, rad_q;
@@ -130,16 +123,14 @@ inline bool fft_make_rader_plan(int n, int r, int pr, bool column_layout, HostFf
     if (r == 1) rad_r.clear();
     if ((int)(rad_r.size() + rad_q.size()) > FFT_MAX_STAGES || n > 32767) return false;
     p.M = n;
-    p.alloc = (column_layout && variant == 1) ? 2 * n : n;
     p.bluestein = 0;
-    p.rader = variant;
+    p.rader = 1;
     p.rr = r; p.rp = pr; p.rq = q;
     p.nouter = (int)rad_r.size();
     p.nfac = p.nouter + (int)rad_q.size();
     p.pad = 0;
-    p.mag_rp = fft_magic((unsigned)pr);
     int prod = 1;
-    for (int s = 0; s < p.nouter; ++s) {               // DIF on length n
+    for (int s = 0; s < p.nouter; ++s) {               // DIT on length n (butterfly stride m_s as for DIF)
         p.fac[s] = rad_r[s];
         prod *= rad_r[s];
         p.sub[s] = n / prod;
@@ -206,58 +197,37 @@ inline bool fft_make_rader_plan(int n, int r, int pr, bool column_layout, HostFf
         const std::complex<double> v = bk[subperm[pos]] / (double)q;
         H.bhat[pos] = make_float2((float)v.real(), (float)v.imag());
     }
-    // where every output lands: block position -> k1 (digits of the outer DIF network), slot -> k2; natural k = k1 + r * k2
+    // input i = sum_s d_s prod_{t<s} fac_t + r * j sits at position sum_s d_s sub_s + slot(j); the radix stages of r then run over
+    // blocks that hold their spectra in generator order, so X[k2 + rp * K1] ends at position K1 * rp + slot(k2)
+    std::vector<int> k2_of_slot(pr, 0);                // slot 1 + m holds X[g^-m]
+    for (int m = 0; m < q; ++m) k2_of_slot[1 + m] = gpow[(q - m) % q];
+    H.pos_in.assign(n, 0);
+    for (int i = 0; i < n; ++i) {
+        int rem = i % r, pos = 0;
+        for (int s = 0; s < p.nouter; ++s) { pos += (rem % p.fac[s]) * p.sub[s]; rem /= p.fac[s]; }
+        H.pos_in[i] = (unsigned short)(pos + H.pin[i / r]);
+    }
     H.perm.assign(n, 0);
     H.inv.assign(n, 0);
-    for (int blk = 0; blk < r; ++blk) {
-        int rem = blk * pr, k1 = 0, w = 1;
-        for (int s = 0; s < p.nouter; ++s) {
-            const int d = rem / p.sub[s];
-            rem -= d * p.sub[s];
-            k1 += d * w;
-            w *= p.fac[s];
-        }
-        for (int slot = 0; slot < pr; ++slot) {
-            const int k2 = slot == 0 ? 0 : gpow[(q - (slot - 1)) % q];             // slot 1 + m holds X[g^-m]
-            const int k = k1 + r * k2;
-            H.perm[blk * pr + slot] = (unsigned short)k;
-            H.inv[k] = (unsigned short)(blk * pr + slot);
-        }
-    }
-    H.pos_in.clear();
-    if (variant == 2) {
-        // decimation in time: input i = sum_s d_s prod_{t<s} fac_t + r * j sits at position sum_s d_s sub_s + slot(j); the radix stages of
-        // r then run over blocks that hold their spectra in generator order, so X[k2 + rp * K1] ends at position K1 * rp + slot(k2)
-        std::vector<int> slot_of_k2(pr, 0), k2_of_slot(pr, 0);
-        for (int m = 0; m < q; ++m) { const int k2 = gpow[(q - m) % q]; slot_of_k2[k2] = 1 + m; k2_of_slot[1 + m] = k2; }
-        H.pos_in.assign(n, 0);
-        for (int i = 0; i < n; ++i) {
-            int rem = i % r, pos = 0;
-            for (int s = 0; s < p.nouter; ++s) { pos += (rem % p.fac[s]) * p.sub[s]; rem /= p.fac[s]; }
-            H.pos_in[i] = (unsigned short)(pos + H.pin[i / r]);
-        }
-        for (int pos = 0; pos < n; ++pos) {
-            const int k = (pos / pr) * pr + k2_of_slot[pos % pr];
-            H.perm[pos] = (unsigned short)k;
-            H.inv[k] = (unsigned short)pos;
-        }
+    for (int pos = 0; pos < n; ++pos) {
+        const int k = (pos / pr) * pr + k2_of_slot[pos % pr];
+        H.perm[pos] = (unsigned short)k;
+        H.inv[k] = (unsigned short)pos;
     }
     H.chirp.clear();
     return true;
 }
 
-// Build the plan for length n.  stockham = true: out-of-place autosort order for direct lengths (rows).
-inline bool fft_make_plan(int n, bool stockham, HostFftPlan& H) {
+// Build the plan for length n.  stockham = true: out-of-place autosort order for direct lengths (rows).  rader = false: Bluestein
+// for every non-smooth length (lets the host test run the Bluestein code on the lengths Rader would take).
+inline bool fft_make_plan(int n, bool stockham, HostFftPlan& H, bool rader = true) {
     FftPlan& p = H.p;
     p = FftPlan{};
     p.n = n;
     std::vector<int> rad;
     {
         int rr = 0, rp = 0;
-        // `stockham` is what the callers pass for the sequence-major (row) layout; the column layout needs the two halves
-        if (fft_rader_enabled() && !fft_radices(n, rad) && fft_rader_split(n, &rr, &rp) &&
-            fft_make_rader_plan(n, rr, rp, !stockham, H, fft_rader_enabled() == 2 ? 2 : 1))
-            return true;
+        if (rader && !fft_radices(n, rad) && fft_rader_split(n, &rr, &rp) && fft_make_rader_plan(n, rr, rp, H)) return true;
         p = FftPlan{};
         p.n = n;
     }
@@ -284,7 +254,6 @@ inline bool fft_make_plan(int n, bool stockham, HostFftPlan& H) {
         stockham = false;
     }
     const int M = p.M;
-    p.alloc = M;
     if (M > 65535) return false;
     if (stockham) std::reverse(rad.begin(), rad.end());   // odd radix first: its stride-R stores are conflict free
     p.nfac = (int)rad.size();

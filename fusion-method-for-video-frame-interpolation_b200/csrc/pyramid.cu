@@ -167,17 +167,13 @@ static int get_fft(fvfi_pyr_plan* p, int n, bool stockham, FftPlan* out) {
     f.chirp = nullptr;
     f.bhat = nullptr;
     f.tw2 = nullptr;
-    f.pin = nullptr;
     f.inv = nullptr;
     f.pos_in = nullptr;
-    if (f.rader == 2) {
-        if (int rc = upload(p, H.pos_in, &f.pos_in)) return rc;
-    }
     if (f.rader) {
+        if (int rc = upload(p, H.pos_in, &f.pos_in)) return rc;
         if (int rc = upload(p, H.perm, &f.perm)) return rc;
         if (int rc = upload(p, H.bhat, &f.bhat)) return rc;
         if (int rc = upload(p, H.tw2, &f.tw2)) return rc;
-        if (int rc = upload(p, H.pin, &f.pin)) return rc;
         if (int rc = upload(p, H.inv, &f.inv)) return rc;
     } else if (f.bluestein) {
         if (int rc = upload(p, H.chirp, &f.chirp)) return rc;
@@ -191,8 +187,8 @@ static int get_fft(fvfi_pyr_plan* p, int n, bool stockham, FftPlan* out) {
 }
 
 static size_t row_bytes_per_row(const FftPlan& fx) {
-    // Bluestein and Rader (decimation in time) run in place; Stockham and the decimation-in-frequency Rader variant use two buffers
-    return (size_t)((fx.bluestein || fx.rader == 2) ? 1 : 2) * fft_pitch(fx) * sizeof(float2);
+    // Bluestein and Rader run in place; Stockham uses two buffers
+    return (size_t)((fx.bluestein || fx.rader) ? 1 : 2) * fft_pitch(fx) * sizeof(float2);
 }
 
 static int build_jobs(fvfi_pyr_plan* p) {
@@ -214,8 +210,8 @@ static int build_jobs(fvfi_pyr_plan* p) {
         if (int rc = get_fft(p, J.h, false, &J.fy)) return rc;
         if (int rc = get_fft(p, J.w, true, &J.fx)) return rc;
         int cs = 3;
-        while (cs > 0 && ((size_t)J.fy.alloc << cs) * sizeof(float2) > COL_SMEM_MAX) --cs;
-        if (((size_t)J.fy.alloc << cs) * sizeof(float2) > 220 * 1024) { set_error("pyramid: column length %d too large", J.h); return FVFI_EINVAL; }
+        while (cs > 0 && ((size_t)J.fy.M << cs) * sizeof(float2) > COL_SMEM_MAX) --cs;
+        if (((size_t)J.fy.M << cs) * sizeof(float2) > 220 * 1024) { set_error("pyramid: column length %d too large", J.h); return FVFI_EINVAL; }
         J.ct_shift = cs;
         const size_t per_row = row_bytes_per_row(J.fx);
         if (per_row > 220 * 1024) { set_error("pyramid: row length %d too large", J.w); return FVFI_EINVAL; }
@@ -224,7 +220,7 @@ static int build_jobs(fvfi_pyr_plan* p) {
         J.rb = rb;
         J.col_tiles = ceil_div(J.w, 1 << cs);
         int cc = cs;                 // combine pass: transform buffer + accumulator, aim for three CTAs per SM
-        while (cc > 2 && (((size_t)J.fy.alloc + J.h) << cc) * sizeof(float2) > 75 * 1024) --cc;
+        while (cc > 2 && (((size_t)J.fy.M + J.h) << cc) * sizeof(float2) > 75 * 1024) --cc;
         J.ct_shift_c = cc;
         J.col_tiles_c = ceil_div(J.w, 1 << cc);
         J.row_tiles = ceil_div(J.h, rb);
@@ -565,7 +561,7 @@ __global__ void __launch_bounds__(PYR_THREADS, PYR_MIN_CTAS) k_cols_fwd(const Le
     const int E_ = h << cs;
     const FftIO ioy = fft_io(J.fy);
     float2* a = smem;
-    float2* acc = smem + ((size_t)J.fy.alloc << cs);
+    float2* acc = smem + ((size_t)J.fy.M << cs);
     const size_t plane = (size_t)h * w;
     const FftCtx cx{(int)threadIdx.x, (int)blockDim.x};
     FftResult R{a, nullptr};
@@ -861,7 +857,7 @@ static int ensure_smem(K kernel, size_t bytes) {
 
 static size_t row_smem(const LevelJob& J) { return (size_t)J.rb * row_bytes_per_row(J.fx) + 16; }   // + the mbarrier of the bulk row loads
 static size_t col_smem(const LevelJob& J, bool combine) {
-    return combine ? ((((size_t)J.fy.alloc + J.h) << J.ct_shift_c) * sizeof(float2)) : (((size_t)J.fy.alloc << J.ct_shift) * sizeof(float2));
+    return combine ? ((((size_t)J.fy.M + J.h) << J.ct_shift_c) * sizeof(float2)) : (((size_t)J.fy.M << J.ct_shift) * sizeof(float2));
 }
 
 struct SetBuilder {
@@ -1170,7 +1166,6 @@ int fvfi_pyr_plan_create(int H, int W, int height, int nbands, double scale_fact
     FVFI_CHECK_ARG(height >= 2 && height - 2 < MAX_LEVELS - 1, "pyr_plan_create: bad height %d", height);
     FVFI_CHECK_ARG(nbands >= 1 && nbands <= MAX_BANDS, "pyr_plan_create: nbands must be 1..%d", MAX_BANDS);
     FVFI_CHECK_ARG(scale_factor > 1.0 && scale_factor <= 4.0, "pyr_plan_create: scale_factor must be in (1,4]");
-    if (const char* e = getenv("FVFI_FFT_NO_RADER")) fvfi::fft_rader_enabled() = (e[0] == '1') ? 0 : (e[0] == '2') ? 1 : 2;   // A/B switch: 1 = Bluestein everywhere, 2 = Rader with the permuting copy
     fvfi_pyr_plan* p = new fvfi_pyr_plan();
     p->H = H; p->W = W; p->height = height; p->nbands = nbands; p->L = height - 2; p->scale = scale_factor;
     if (int rc = build_plan(p)) { fvfi_pyr_plan_destroy(p); return rc; }

@@ -114,7 +114,7 @@ class KernelEstimation(torch.nn.Module):
                 i += 3 if act else 2
             elif isinstance(m, torch.nn.Upsample):
                 size = (x.shape[2] * 2, x.shape[3] * 2)
-                if (tc.fuse_upsample and m.mode == 'bilinear' and m.scale_factor == 2 and i + 1 < len(mods)
+                if (m.mode == 'bilinear' and m.scale_factor == 2 and i + 1 < len(mods)
                         and isinstance(mods[i + 1], torch.nn.Conv2d) and mods[i + 1].kernel_size[0] > 1):
                     up = (size, bool(m.align_corners))      # Upsample -> Conv2d: one kernel (fvfi_conv2d_nhwc_upsampled)
                 else:

@@ -201,9 +201,6 @@ def to_nhwc(x):
     return x.contiguous(memory_format=torch.channels_last)
 
 
-fuse_upsample = True    # Upsample -> Conv2d as one kernel (A/B switch for tools/; the unfused form is resize_bilinear + conv2d)
-
-
 def conv2d(x, weight, bias=None, padding_mode="zeros", act=None, out=None, nchw_out=False, pad_out=False, residual=None,
            upsample=None, x_direct=None):
     """x [B,Cin,H,W] (any memory format; channels_last avoids a copy) -> [B,Cout,H,W] channels_last

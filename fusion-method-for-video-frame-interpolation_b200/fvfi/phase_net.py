@@ -209,33 +209,21 @@ class PhaseNet(nn.Module):
                 l = L - 1 - idx                                                            # coarsest level first
                 ph, am = vals.phase[l], vals.amplitude[l]
                 h, w = int(ph.shape[2]), int(ph.shape[3])
-                cf, cp, cv = feature.shape[1], prediction.shape[1], 2 * nb
+                cp, cv = prediction.shape[1], 2 * nb
                 i = idx + 1 if idx + 1 < len(self.layers) - 1 else len(self.layers) - 1
-                if tc.fuse_upsample and cf % 32 == 0:
-                    # cat(interpolate(feature), values, interpolate(prediction)) is never built: the value channels and the resampled
-                    # prediction go into a compact [.., 24] record, the 64 feature channels are resampled by the loaders of the
-                    # level's first convolution
-                    cd = (2 * cv + cp + 7) // 8 * 8
-                    direct = torch.empty((pc, cd, h, w), dtype=torch.float32, device=dev, memory_format=torch.channels_last)
-                    if cd != 2 * cv + cp:
-                        direct.zero_()                                                     # padding channels must be finite
-                    with torch.cuda.device(dev):
-                        _lib.check(lib.fvfi_phasenet_assemble_offset(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(), direct.data_ptr(),
-                                                                     direct.stride(3), N, P, q, p0, pc, nb, h, w, _lib.stream_ptr()))
-                    tc.resize_bilinear(prediction, (h, w), False, out=direct, out_channel_offset=2 * cv)
-                    feature, prediction = self.layers[i].forward_resampled(feature, direct, (h, w))
-                    del direct
-                else:
-                    concat = torch.empty((pc, cf + 2 * cv + cp, h, w), dtype=torch.float32, device=dev,
-                                         memory_format=torch.channels_last)
-                    tc.resize_bilinear(feature, (h, w), False, out=concat, out_channel_offset=0)
-                    with torch.cuda.device(dev):
-                        _lib.check(lib.fvfi_phasenet_assemble_offset(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(),
-                                                                     concat.data_ptr() + 4 * cf, concat.stride(3), N, P, q, p0, pc, nb,
-                                                                     h, w, _lib.stream_ptr()))
-                    tc.resize_bilinear(prediction, (h, w), False, out=concat, out_channel_offset=cf + 2 * cv)
-                    feature, prediction = self.layers[i](concat)
-                    del concat
+                # cat(interpolate(feature), values, interpolate(prediction)) is never built: the value channels and the resampled
+                # prediction go into a compact [.., 24] record, the 64 feature channels are resampled by the loaders of the
+                # level's first convolution
+                cd = (2 * cv + cp + 7) // 8 * 8
+                direct = torch.empty((pc, cd, h, w), dtype=torch.float32, device=dev, memory_format=torch.channels_last)
+                if cd != 2 * cv + cp:
+                    direct.zero_()                                                         # padding channels must be finite
+                with torch.cuda.device(dev):
+                    _lib.check(lib.fvfi_phasenet_assemble_offset(ph.data_ptr(), am.data_ptr(), den[l].data_ptr(), direct.data_ptr(),
+                                                                 direct.stride(3), N, P, q, p0, pc, nb, h, w, _lib.stream_ptr()))
+                tc.resize_bilinear(prediction, (h, w), False, out=direct, out_channel_offset=2 * cv)
+                feature, prediction = self.layers[i].forward_resampled(feature, direct, (h, w))
+                del direct
                 pr = tc.to_nhwc(prediction)
                 with torch.cuda.device(dev):
                     _lib.check(lib.fvfi_phasenet_outputs_offset(pr.data_ptr(), pr.stride(3), am.data_ptr(), phase_out[l].data_ptr(),

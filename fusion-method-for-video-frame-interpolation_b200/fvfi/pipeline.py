@@ -69,8 +69,6 @@ class FusionPipeline(torch.nn.Module):
         self.stages = None  # set to a dict to capture intermediates (tests)
         self.max_batch = 8  # frame pairs per sub-batch at full HD (see forward)
         self.timing = None  # set to a list to collect (stage, start_event, end_event) (bench)
-        self.fused_phase_glue = True   # PhaseNet.forward_fused (False: the reference's step-by-step value plumbing)
-        self.pair_baseline = True      # baseline passes 2 and 3 (interpolate_twoframe.py:229,233) as one AdaCoFNet call on 2B frames
         self.max_batch_adacof = 16     # largest AdaCoFNet batch at full HD (the 64 -> 448 fused head tensor is 15 GB at 16)
         self._copy_streams = None      # (host -> device, device -> host) side streams of interpolate_host
         self._graphs = {}              # (method, input shapes) -> GraphedCall
@@ -164,14 +162,9 @@ class FusionPipeline(torch.nn.Module):
         # PhaseNet branch (:168-192)
         vals = self._filter("phasenet", planes, want_high=False)
         self._tick('pyr.filter(12 planes/frame)')
-        if self.fused_phase_glue:
-            # separate_vals / get_concat_layers_inf / normalize_vals / forward / reverse_normalize with the regrouping and the
-            # (de)normalisation fused into the concat assembly and the output kernel (PhaseNet.forward_fused)
-            vals_pred = self.phase_net.forward_fused(vals, pyr.last_amp_max, frame2=q)
-        else:
-            vals_in = self.phase_net.normalize_vals(utils.get_concat_layers_inf(pyr, utils.pair_vals(vals, q, pyr.nbands)))
-            vals_pred = self.phase_net(vals_in)
-            del vals_in
+        # separate_vals / get_concat_layers_inf / normalize_vals / forward / reverse_normalize with the regrouping and the
+        # (de)normalisation fused into the concat assembly and the output kernel (PhaseNet.forward_fused)
+        vals_pred = self.phase_net.forward_fused(vals, pyr.last_amp_max, frame2=q)
         del vals
         self._tick('phase_net')
         lab_pred = pyr.inv_filter_sparse(vals_pred, use_high=False).reshape(r_shape)            # high_level is zeros (:127-128)
@@ -188,24 +181,15 @@ class FusionPipeline(torch.nn.Module):
             # only level 0 + the high residual (h_freq) and the six coarsest levels + low pass (freq_diff) of these pyramids are ever read
             L = pyr.height - 2
             coarse = list(range(L - 6, L))
-            if self.fused_phase_glue:
-                # h_freq - h_freq_ph = mean_c(recon_{high + level 0}(ada_c) - recon_{high + level 0}(phase_c))  (get_last_value_levels(., 1),
-                # :205-209).  Decomposition and reconstruction are linear in the image, so this is recon_{high + level 0} of the single
-                # plane  xbar = mean_c(ada_c - phase_c): the six colour planes are decomposed on the (tiny) coarse levels only.
-                vals_ada, vals_ph = utils.separate_vals(
-                    self._filter("uncertainty", torch.cat((ada_pred.reshape(-1, H, W), phase_pred.reshape(-1, H, W)), 0), want_high=False,
-                                 levels=coarse), 2)
-                self._tick('lab2rgb+pyr.filter(6 planes/frame)')
-                # ... and recon_{high + level 0}(D(x)) is a linear filter of x: one spectral multiplication (Pyramid.highband_filter)
-                h_diff = pyr.highband_filter((ada_pred - phase_pred).mean(1))
-            else:
-                used = sorted(set([0]) | set(coarse))
-                vals_ada, vals_ph = utils.separate_vals(
-                    self._filter("uncertainty", torch.cat((ada_pred.reshape(-1, H, W), phase_pred.reshape(-1, H, W)), 0), levels=used), 2)
-                self._tick('lab2rgb+pyr.filter(6 planes/frame)')
-                h_freq = pyr.inv_filter_sparse(vals_ada, use_low=False, levels=[0]).reshape(r_shape).mean(1)
-                h_freq_ph = pyr.inv_filter_sparse(vals_ph, use_low=False, levels=[0]).reshape(r_shape).mean(1)
-                h_diff = h_freq - h_freq_ph
+            # h_freq - h_freq_ph = mean_c(recon_{high + level 0}(ada_c) - recon_{high + level 0}(phase_c))  (get_last_value_levels(., 1),
+            # :205-209).  Decomposition and reconstruction are linear in the image, so this is recon_{high + level 0} of the single
+            # plane  xbar = mean_c(ada_c - phase_c): the six colour planes are decomposed on the (tiny) coarse levels only.
+            vals_ada, vals_ph = utils.separate_vals(
+                self._filter("uncertainty", torch.cat((ada_pred.reshape(-1, H, W), phase_pred.reshape(-1, H, W)), 0), want_high=False,
+                             levels=coarse), 2)
+            self._tick('lab2rgb+pyr.filter(6 planes/frame)')
+            # ... and recon_{high + level 0}(D(x)) is a linear filter of x: one spectral multiplication (Pyramid.highband_filter)
+            h_diff = pyr.highband_filter((ada_pred - phase_pred).mean(1))
             h_freq_diff = (h_diff.abs() * 100).clamp(min=0, max=1.0)
             self._tick('pyr.inv_filter(level0 x2)')
             phase_uncertainty = filters.gaussian_filter(h_freq_diff, 5)
@@ -231,7 +215,7 @@ class FusionPipeline(torch.nn.Module):
         else:
             phase_uncertainty, ada_uncertainty, freq_diff, h_freq_diff = uncertainty_maps()
         # baseline (:228-238)
-        if self.pair_baseline and 2 * B <= self.max_batch_adacof:
+        if 2 * B <= self.max_batch_adacof:
             # passes 2 and 3 (:229, :233) are independent: ONE AdaCoFNet call on a 2B batch (twice the tiles for the coarse layers)
             inb = self.adacof(torch.cat((rgb1, phase_pred), 0), torch.cat((phase_pred, rgb2), 0), return_warped=False, want_mask=False)[2]
             inb1, inb2 = inb[:B], inb[B:]
@@ -265,10 +249,7 @@ class FusionPipeline(torch.nn.Module):
         pyr = self.pyr
         lab1, lab2 = transform.rgb2lab(rgb1), transform.rgb2lab(rgb2)
         vals = self._filter("phasenet", torch.cat((lab1.reshape(-1, H, W), lab2.reshape(-1, H, W)), 0), want_high=False)
-        if self.fused_phase_glue:
-            vals_pred = self.phase_net.forward_fused(vals, pyr.last_amp_max)
-        else:
-            vals_pred = self.phase_net(self.phase_net.normalize_vals(utils.get_concat_layers_inf(pyr, utils.separate_vals(vals, 2))))
+        vals_pred = self.phase_net.forward_fused(vals, pyr.last_amp_max)
         lab_pred = pyr.inv_filter_sparse(vals_pred, use_high=False).reshape(B, 3, H, W)
         phase_pred = transform.lab2rgb(lab_pred)
         if self.stages is not None:

@@ -38,19 +38,6 @@ def separate_vals(vals, num_input):
     return out
 
 
-def pair_vals(vals, q, nbands):
-    """The two per-frame DecompValues of a decomposition in which frame 2 of pair-plane p is plane p + q (views): frame 1 = planes
-    [0, P), frame 2 = planes [q, q + P), P = N - q.  q = N / 2 is ``separate_vals(vals, 2)``; q = 3 is a clip of consecutive
-    frames decomposed once (pair t = frames t, t + 1)."""
-    N = vals.low_level.shape[0]
-    P = N - q
-    planes = lambda t, k: t[k:k + P]
-    bands = lambda t, k: None if t is None else t[k * nbands:(k + P) * nbands]
-    return [DecompValues(high_level=planes(vals.high_level, k), low_level=planes(vals.low_level, k),
-                         phase=[bands(p, k) for p in vals.phase], amplitude=[bands(a, k) for a in vals.amplitude])
-            for k in (0, q)]
-
-
 def combine_values(vals_list):
     """utils.py:208-240."""
     return DecompValues(

@@ -9,11 +9,12 @@
 using namespace fvfi;
 
 // mode 0: rows layout, out-of-place (Stockham) for direct lengths; mode 1: columns layout, in-place DIF (+perm)
+// rader 0: Bluestein for every non-smooth length (fft_make_plan's rader = false); otherwise the plans the library uses.
 // in/out: [batch][n][2] floats.  Returns 0, or -1 if no plan.
-extern "C" int fft_host_run(int n, int mode, int batch, const float* in, float* out, int* info) {
+extern "C" int fft_host_run(int n, int mode, int batch, const float* in, float* out, int* info, int rader) {
     HostFftPlan H;
     const bool col = mode == 1;
-    if (!fft_make_plan(n, !col, H)) return -1;
+    if (!fft_make_plan(n, !col, H, rader != 0)) return -1;
     H.p.tw = H.tw.data();
     H.p.perm = H.p.bluestein ? nullptr : H.perm.data();
     H.p.chirp = H.chirp.data();
@@ -21,17 +22,16 @@ extern "C" int fft_host_run(int n, int mode, int batch, const float* in, float* 
     if (H.p.rader) {
         H.p.perm = H.perm.data();
         H.p.tw2 = H.tw2.data();
-        H.p.pin = H.pin.data();
         H.p.inv = H.inv.data();
-        H.p.pos_in = H.pos_in.empty() ? nullptr : H.pos_in.data();
+        H.p.pos_in = H.pos_in.data();
     }
     const int M = H.p.M;
     int ctshift = 0;
     while ((1 << ctshift) < batch) ++ctshift;
     const int pitch = fft_pitch(H.p);
-    const size_t elems = col ? ((size_t)H.p.alloc << ctshift) : (size_t)batch * pitch;
+    const size_t elems = col ? ((size_t)M << ctshift) : (size_t)batch * pitch;
     // garbage-filled on purpose, with a guard zone behind each buffer: the stage code must stay inside [0, elems) -- the bound the
-    // kernels size their shared memory by (alloc << ctshift columns / batch * pitch rows)
+    // kernels size their shared memory by (M << ctshift columns / batch * pitch rows)
     constexpr size_t GUARD = 256;
     const float2 canary = make_float2(-12345.f, 54321.f);
     std::vector<float2> a(elems + GUARD, make_float2(7.f, 7.f)), b(elems + GUARD, make_float2(9.f, 9.f));
@@ -56,11 +56,8 @@ extern "C" int fft_host_run(int n, int mode, int batch, const float* in, float* 
     if (info) {
         info[0] = M;
         info[1] = H.p.bluestein + 2 * (H.p.rader != 0);
-        info[15] = H.p.rader;
         info[2] = H.p.nfac;
         for (int s = 0; s < H.p.nfac; ++s) info[3 + s] = H.p.fac[s];
     }
     return 0;
 }
-
-extern "C" void fft_host_set_rader(int on) { fft_rader_enabled() = on; }

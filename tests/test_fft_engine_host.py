@@ -25,7 +25,7 @@ def lib():
         subprocess.check_call(["nvcc", "-O1", "-std=c++17", "-shared", "-Xcompiler", "-fPIC", "-Wno-deprecated-gpu-targets",
                                "-I", CSRC, "-o", SO, SRC])
     L = ctypes.CDLL(SO)
-    L.fft_host_run.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
+    L.fft_host_run.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
     return L
 
 
@@ -37,11 +37,11 @@ def level_lengths(n, levels):
     return out
 
 
-def run(L, n, mode, batch, rng):
+def run(L, n, mode, batch, rng, rader=True):
     x = (rng.standard_normal((batch, n)) + 1j * rng.standard_normal((batch, n))).astype(np.complex64)
     out = np.zeros((batch, n), np.complex64)
     info = np.zeros(16, np.int32)
-    rc = L.fft_host_run(n, mode, batch, x.ctypes.data, out.ctypes.data, info.ctypes.data)
+    rc = L.fft_host_run(n, mode, batch, x.ctypes.data, out.ctypes.data, info.ctypes.data, int(rader))
     assert rc != -2, "n=%d mode=%d: the transform wrote outside its buffers (guard zone overwritten)" % (n, mode)
     assert rc == 0, "no plan for n=%d" % n
     ref = np.fft.fft(x.astype(np.complex128), axis=1)
@@ -55,29 +55,23 @@ LENGTHS = sorted(set(
     + level_lengths(2160, 18) + level_lengths(3840, 18)))
 
 
-@pytest.mark.parametrize("rader", [2, 1, 0])
+@pytest.mark.parametrize("rader", [True, False], ids=["2", "0"])      # ids: 2 = the shipped plans, 0 = Bluestein only
 @pytest.mark.parametrize("mode", [0, 1])
 def test_all_lengths(lib, mode, rader):
-    """rader = 2: the shipped plans (Rader, decimation in time, for n = r * p with p - 1 smooth; Bluestein for the rest); rader = 1:
-    the decimation-in-frequency Rader variant (permuting copy, two buffers); rader = 0: Bluestein for every non-smooth length -- the
-    alternative paths stay tested."""
-    lib.fft_host_set_rader(rader)
+    """rader = True: the shipped plans (Rader for n = r * p with p - 1 smooth; Bluestein for the rest); rader = False: Bluestein for
+    every non-smooth length -- the Bluestein code runs on many more lengths."""
     rng = np.random.default_rng(mode)
     worst, kinds = 0.0, {0: 0, 1: 0, 2: 0}
-    try:
-        for n in LENGTHS:
-            batch = 2 if n > 512 else 4
-            err, info = run(lib, n, mode, batch, rng)
-            kinds[int(info[1])] += 1
-            assert info[1] != 2 or info[15] == rader, "n=%d: asked for Rader variant %d, plan is variant %d" % (n, rader, info[15])
-            tol = 4e-6 if info[1] else 2e-6      # Bluestein: two FFTs of ~2n + chirps; Rader: two FFTs of p - 1 + the outer stages
-            assert err < tol, "n=%d mode=%d rel err %.3g (M=%d kind=%d radices=%s)" % (
-                n, mode, err, info[0], info[1], list(info[3:3 + info[2]]))
-            worst = max(worst, err)
-    finally:
-        lib.fft_host_set_rader(2)
+    for n in LENGTHS:
+        batch = 2 if n > 512 else 4
+        err, info = run(lib, n, mode, batch, rng, rader)
+        kinds[int(info[1])] += 1
+        tol = 4e-6 if info[1] else 2e-6      # Bluestein: two FFTs of ~2n + chirps; Rader: two FFTs of p - 1 + the outer stages
+        assert err < tol, "n=%d mode=%d rel err %.3g (M=%d kind=%d radices=%s)" % (
+            n, mode, err, info[0], info[1], list(info[3:3 + info[2]]))
+        worst = max(worst, err)
     print("worst relative error", worst, "plans direct/bluestein/rader:", kinds)
-    assert (kinds[2] > 10) == bool(rader)
+    assert (kinds[2] > 10) == rader
 
 
 def test_plan_choices(lib):

@@ -149,19 +149,32 @@ def test_phasenet_256_vs_reference_golden(golden_dir, fused):
     """BASELINE.json configs[0]: PhaseNet decompose -> predict -> reconstruct on one 256x256 frame pair, random-init weights, against
     the reference's own Pyramid wrapper + PhaseNet on CPU (tests/golden/phasenet_ref_256x256_s5.npz): every predicted level
     (as complex coefficients), the low pass, the reconstructed Lab planes and the RGB frame.  Pyramid(12, 4, sqrt 2):
-    levels 256,181,128,91,64,45,32,23,16,11 + low 8 -> layers[7] (phase_net.py:148) serves the four finest levels."""
+    levels 256,181,128,91,64,45,32,23,16,11 + low 8 -> layers[7] (phase_net.py:148) serves the four finest levels.
+    fused: FusionPipeline.phase_interp (PhaseNet.forward_fused); not fused: the stepwise module API (separate_vals ->
+    get_concat_layers_inf -> normalize_vals -> PhaseNet.forward) on the same decomposition."""
     from _parity import WrapAligner, fmt, stage_report
+    from fvfi import transform, utils
     from fvfi.pipeline import FusionPipeline
     z = np.load(os.path.join(golden_dir, "phasenet_ref_256x256_s5.npz"))
     B, H, W, seed = [int(v) for v in z["meta"]]
     pipe = FusionPipeline(H, W, "cuda")
     assert pipe.pyr.height == 12
     pipe.load_state(_state_for(z, seed))
-    pipe.fused_phase_glue = fused
     pipe.filter_hook = al = WrapAligner(z)                    # compare on the reference's branch of the wrapped input phases
     pipe.stages = {}
     rgb1, rgb2 = fp.seeded_frames(B, H, W, seed)
-    pipe.phase_interp(rgb1.cuda(), rgb2.cuda())
+    if fused:
+        pipe.phase_interp(rgb1.cuda(), rgb2.cuda())
+    else:
+        pyr, net = pipe.pyr, pipe.phase_net
+        with torch.no_grad():
+            lab1, lab2 = transform.rgb2lab(rgb1.cuda()), transform.rgb2lab(rgb2.cuda())
+            vals = pipe._filter("phasenet", torch.cat((lab1.reshape(-1, H, W), lab2.reshape(-1, H, W)), 0), want_high=False)
+            vals_pred = net(net.normalize_vals(utils.get_concat_layers_inf(pyr, utils.separate_vals(vals, 2))))
+            lab_pred = pyr.inv_filter_sparse(vals_pred, use_high=False).reshape(B, 3, H, W)
+            pipe.stages.update(lab_pred=lab_pred, phase_pred=transform.lab2rgb(lab_pred), low_level=vals_pred.low_level)
+            for l, (p, a) in enumerate(zip(vals_pred.phase, vals_pred.amplitude)):
+                pipe.stages["phase%d" % l], pipe.stages["amp%d" % l] = p, a
     rep = stage_report(z, pipe.stages)
     print("fused" if fused else "stepwise", "wrap flips aligned: %d of %d" % (al.flips, al.coefficients), fmt(rep))
     assert al.flips <= 1e-5 * al.coefficients

@@ -175,16 +175,16 @@ def _count_excess(a, b, tol):
 
 
 @gpu
-@pytest.mark.parametrize("fused", [True, False])
+@pytest.mark.parametrize("concurrent_small", [True, False])
 @pytest.mark.parametrize("H,W,T,mb", [(64, 96, 6, 2), (256, 256, 5, 3), (184, 328, 4, 8)])
-def test_interpolate_sequence_matches_pairs(H, W, T, mb, fused):
+def test_interpolate_sequence_matches_pairs(H, W, T, mb, concurrent_small):
     """The clip path (each frame converted and decomposed once per window, glue in the q = 3 layout) against the pair path on
-    frames[:-1], frames[1:] with the same sub-batching."""
+    frames[:-1], frames[1:] with the same sub-batching, with and without the side-stream fork of small frames."""
     from fvfi import synth
     pipe = _pipe(H, W, seed=2, max_batch=mb)
-    pipe.fused_phase_glue = fused
     if H * W <= 512 * 512:
         assert pipe.concurrent_small                        # 64x96 and 256x256 take the side-stream fork
+    pipe.concurrent_small = concurrent_small
     clip = synth.seeded_clip(T, H, W, 5, shift=(2, -3)).cuda()
     got = pipe.interpolate_sequence(clip)
     want = pipe(clip[:-1], clip[1:])

@@ -97,12 +97,10 @@ with torch.no_grad():
     print("C  reconstruction of the oracle's prediction: max abs vs oracle fp32 %.2e ; oracle fp32 vs fp64 (own values) %.2e"
           % (float((rec - o32["rec"]).abs().max()), float((o32["rec"].double() - o64["rec"]).abs().max())))
     # ---- D: whole branch
-    for fused in (True, False):
-        pipe.fused_phase_glue = fused
-        pipe.stages = {}
-        pipe.phase_interp(rgb1.cuda(), rgb2.cuda())
-        lp = pipe.stages["lab_pred"].reshape(-1, H, W).cpu()
-        print("D  whole branch (%s): lab_pred max abs vs oracle fp32 %.2e, vs fp64 %.2e ; oracle fp32 vs fp64 %.2e"
-              % ("fused" if fused else "stepwise", float((lp - o32["rec"]).abs().max()), float((lp.double() - o64["rec"]).abs().max()),
-                 float((o32["rec"].double() - o64["rec"]).abs().max())))
-        pipe.stages = None
+    pipe.stages = {}
+    pipe.phase_interp(rgb1.cuda(), rgb2.cuda())
+    lp = pipe.stages["lab_pred"].reshape(-1, H, W).cpu()
+    print("D  whole branch: lab_pred max abs vs oracle fp32 %.2e, vs fp64 %.2e ; oracle fp32 vs fp64 %.2e"
+          % (float((lp - o32["rec"]).abs().max()), float((lp.double() - o64["rec"]).abs().max()),
+             float((o32["rec"].double() - o64["rec"]).abs().max())))
+    pipe.stages = None
