@@ -19,6 +19,7 @@
 #include <cstdlib>
 
 #include "common.cuh"
+#include "yuv.cuh"
 
 namespace fvfi {
 
@@ -475,6 +476,51 @@ __global__ void __launch_bounds__(256) fusion_blend_rgb8_kernel(const float* __r
         dst[c] = (uint8_t)__float2uint_rn(fusion_blend_px(__ldcs(base + o + c * plane), __ldcs(x + o + c * plane)) * 255.f);
 }
 
+// An 8-bit code from a value on the 0..255 scale: clamp, then round half to even.
+__device__ __forceinline__ uint8_t code8(float v) { return (uint8_t)__float2uint_rn(fminf(fmaxf(v, 0.f), 255.f)); }
+
+// Y' = (Kr R' + Kg G') + Kb B', every product and sum rounded on its own (no FMA contraction).
+__device__ __forceinline__ float luma(float r, float g, float b, const YuvCoeffs& k) {
+    return __fadd_rn(__fadd_rn(__fmul_rn(k.kr, r), __fmul_rn(k.kg, g)), __fmul_rn(k.kb, b));
+}
+
+// The same blend for frames that leave as yuv420p [B,3H/2,W] uint8 (include/fvfi.h, fvfi_fusion_blend_yuv420p; oracle/yuv.py restates
+// the arithmetic): one thread owns a 2x2 luma block, blends its 4 pixels x 3 channels (float2 __ldcs loads of both rows), writes the
+// two uchar2 Y pairs, and Cb / Cr of the block's mean R'G'B' (centre-sited chroma).  The fp32 frame is never stored.
+__global__ void __launch_bounds__(256) fusion_blend_yuv420p_kernel(const float* __restrict__ base, const float* __restrict__ x,
+                                                                   uint8_t* __restrict__ out, int H, int W, YuvCoeffs k) {
+    const int Hc = H / 2, Wc = W / 2;
+    const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = blockIdx.y;
+    if (q >= (size_t)Hc * Wc) return;
+    const int i = (int)(q / Wc), j = (int)(q - (size_t)i * Wc);
+    const size_t plane = (size_t)H * W;
+    uint8_t* Y = out + (size_t)n * plane * 3 / 2;
+    float v[3][2][2];                                // [channel][row][column]
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy) {
+        const size_t o = (size_t)(2 * i + dy) * W + 2 * j;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const size_t f = ((size_t)n * 3 + c) * plane + o;
+            const float2 b2 = __ldcs(reinterpret_cast<const float2*>(base + f)), x2 = __ldcs(reinterpret_cast<const float2*>(x + f));
+            v[c][dy][0] = fusion_blend_px(b2.x, x2.x);
+            v[c][dy][1] = fusion_blend_px(b2.y, x2.y);
+        }
+        uchar2 yy;
+        yy.x = code8(__fadd_rn(k.yoff, __fmul_rn(k.ys, luma(v[0][dy][0], v[1][dy][0], v[2][dy][0], k))));
+        yy.y = code8(__fadd_rn(k.yoff, __fmul_rn(k.ys, luma(v[0][dy][1], v[1][dy][1], v[2][dy][1], k))));
+        *reinterpret_cast<uchar2*>(Y + o) = yy;
+    }
+    float m[3];                                      // block mean: ((top-left + top-right) + (bottom-left + bottom-right)) / 4
+#pragma unroll
+    for (int c = 0; c < 3; ++c) m[c] = __fmul_rn(__fadd_rn(__fadd_rn(v[c][0][0], v[c][0][1]), __fadd_rn(v[c][1][0], v[c][1][1])), 0.25f);
+    const float ym = luma(m[0], m[1], m[2], k);
+    const size_t oc = (size_t)i * Wc + j;
+    Y[plane + oc] = code8(__fadd_rn(128.f, __fmul_rn(k.cs, __fmul_rn(__fsub_rn(m[2], ym), k.kCb))));
+    Y[plane + plane / 4 + oc] = code8(__fadd_rn(128.f, __fmul_rn(k.cs, __fmul_rn(__fsub_rn(m[0], ym), k.kCr))));
+}
+
 static int check_dims(int B, int C, int Hin, int Win, int H, int W, int F, int dil) {
     FVFI_CHECK_ARG(B > 0 && C > 0 && H > 0 && W > 0 && F > 0 && dil > 0, "adacof: non-positive dimension");
     // adacof.py:326-327
@@ -673,6 +719,19 @@ extern "C" int fvfi_fusion_blend_rgb8(const float* base, const float* x_pre_tanh
     const size_t plane = (size_t)H * W;
     dim3 grid((unsigned)((plane + 255) / 256), B);
     fusion_blend_rgb8_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(base, x_pre_tanh, out, plane);
+    FVFI_LAUNCH_CHECK();
+    return FVFI_OK;
+}
+
+extern "C" int fvfi_fusion_blend_yuv420p(const float* base, const float* x_pre_tanh, uint8_t* out, int B, int H, int W, int matrix,
+                                         int full_range, void* stream) {
+    FVFI_CHECK_ARG(base && x_pre_tanh && out, "fvfi_fusion_blend_yuv420p: null pointer");
+    if (int rc = yuv_check("fvfi_fusion_blend_yuv420p", B, H, W, matrix, full_range)) return rc;
+    FVFI_CHECK_ARG((uintptr_t)base % 8 == 0 && (uintptr_t)x_pre_tanh % 8 == 0 && (uintptr_t)out % 2 == 0,
+                   "fvfi_fusion_blend_yuv420p: base / x_pre_tanh must be 8-byte and out 2-byte aligned");
+    const size_t blocks = (size_t)(H / 2) * (W / 2);
+    dim3 grid((unsigned)((blocks + 255) / 256), B);
+    fusion_blend_yuv420p_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(base, x_pre_tanh, out, H, W, yuv_coeffs(matrix, full_range));
     FVFI_LAUNCH_CHECK();
     return FVFI_OK;
 }

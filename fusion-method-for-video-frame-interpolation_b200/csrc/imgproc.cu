@@ -4,6 +4,7 @@
 //   k x k median            (scipy.ndimage.median_filter(f, size=50), interpolate_twoframe.py:221-222)
 // Device-resident replacements so the fusion pipeline never leaves the GPU.
 #include "common.cuh"
+#include "yuv.cuh"
 
 namespace fvfi {
 
@@ -18,18 +19,29 @@ __device__ __forceinline__ float lin_to_srgb(float c) {
 __device__ __forceinline__ float lab_f(float t) { return t > 0.008856f ? cbrtf(t) : 7.787f * t + 16.f / 116.f; }
 __device__ __forceinline__ float lab_finv(float f) { return f > 0.2068966f ? f * f * f : (f - 16.f / 116.f) / 7.787f; }
 
-// One pixel: sRGB in [0,1] -> scaled Lab written at dst[0], dst[plane], dst[2*plane] (shared by rgb2lab_kernel and
-// rgb8_to_rgb_lab_kernel, so both give the same bits for the same RGB value).
-__device__ __forceinline__ void rgb_to_scaled_lab(float sr, float sg, float sb, float* dst, size_t plane) {
+// One pixel: sRGB in [0,1] -> scaled Lab (L, a, b) (shared by rgb2lab_kernel, rgb8_to_rgb_lab_kernel and
+// yuv420p_to_rgb_lab_kernel, so all three give the same bits for the same RGB value).
+__device__ __forceinline__ float3 scaled_lab(float sr, float sg, float sb) {
     const float r = srgb_to_lin(sr), g = srgb_to_lin(sg), b = srgb_to_lin(sb);
     const float x = (0.412453f * r + 0.357580f * g + 0.180423f * b) / 0.95047f;
     const float y = (0.212671f * r + 0.715160f * g + 0.072169f * b);
     const float z = (0.019334f * r + 0.119193f * g + 0.950227f * b) / 1.08883f;
     const float fx = lab_f(x), fy = lab_f(y), fz = lab_f(z);
-    dst[0] = (116.f * fy - 16.f) / 100.f;                    // transform.py:9  L / light
-    dst[plane] = (500.f * (fx - fy) + 128.f) / 255.f;        // transform.py:10-11
-    dst[2 * plane] = (200.f * (fy - fz) + 128.f) / 255.f;
+    return make_float3((116.f * fy - 16.f) / 100.f,          // transform.py:9  L / light
+                       (500.f * (fx - fy) + 128.f) / 255.f,  // transform.py:10-11
+                       (200.f * (fy - fz) + 128.f) / 255.f);
 }
+
+// The same, written at dst[0], dst[plane], dst[2*plane].
+__device__ __forceinline__ void rgb_to_scaled_lab(float sr, float sg, float sb, float* dst, size_t plane) {
+    const float3 v = scaled_lab(sr, sg, sb);
+    dst[0] = v.x;
+    dst[plane] = v.y;
+    dst[2 * plane] = v.z;
+}
+
+// An 8-bit code k -> its value k / 255, correctly rounded (__fdiv_rn, not a reciprocal multiply).
+__device__ __forceinline__ float code_value(unsigned k) { return __fdiv_rn((float)k, 255.f); }
 
 __global__ void rgb2lab_kernel(const float* __restrict__ rgb, float* __restrict__ lab, size_t plane, int B) {
     const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -48,13 +60,79 @@ __global__ void __launch_bounds__(256) rgb8_to_rgb_lab_kernel(const uint8_t* __r
     const int n = blockIdx.y;
     if (p >= plane) return;
     const uint8_t* src = rgb8 + ((size_t)n * plane + p) * 3;
-    const float r = __fdiv_rn((float)__ldg(src), 255.f), g = __fdiv_rn((float)__ldg(src + 1), 255.f),
-                b = __fdiv_rn((float)__ldg(src + 2), 255.f);
+    const float r = code_value(__ldg(src)), g = code_value(__ldg(src + 1)), b = code_value(__ldg(src + 2));
     const size_t o = (size_t)n * 3 * plane + p;
     rgb[o] = r;
     rgb[o + plane] = g;
     rgb[o + 2 * plane] = b;
     rgb_to_scaled_lab(r, g, b, lab + o, plane);
+}
+
+// One yuv420p sample -> its 8-bit R'G'B' code (include/fvfi.h, fvfi_yuv420p_to_rgb_lab).  cb16 / cr16 are the 16x chroma of the
+// [1,3]/4 x [1,3]/4 bilinear upsampling.  Every product and sum is rounded on its own (__fmul_rn / __fadd_rn / __fsub_rn: no FMA
+// contraction), in the order oracle/yuv.py restates.
+__device__ __forceinline__ uchar3 yuv_to_rgb_code(int y, int cb16, int cr16, const YuvCoeffs& k) {
+    const float yn = __fdiv_rn((float)y - k.yoff, k.ys);
+    const float cbn = __fdiv_rn((float)(cb16 - 2048), 16.f * k.cs), crn = __fdiv_rn((float)(cr16 - 2048), 16.f * k.cs);
+    const float v[3] = {__fadd_rn(yn, __fmul_rn(k.kR, crn)),
+                        __fsub_rn(__fsub_rn(yn, __fmul_rn(k.kGb, cbn)), __fmul_rn(k.kGr, crn)),
+                        __fadd_rn(yn, __fmul_rn(k.kB, cbn))};
+    unsigned c[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) c[i] = __float2uint_rn(__fmul_rn(fminf(fmaxf(v[i], 0.f), 1.f), 255.f));
+    return make_uchar3(c[0], c[1], c[2]);
+}
+
+// Decoder frames [T,3H/2,W] uint8 (yuv420p: Y [H,W], U [H/2,W/2], V [H/2,W/2] contiguous per frame) -> planar fp32 RGB [T,3,H,W] and
+// planar scaled Lab [T,3,H,W]: the rgb24 frame of the conversion, then exactly rgb8_to_rgb_lab_kernel's k / 255 and Lab.  Chroma is
+// centre-sited: luma row y reads chroma rows i = y/2 and i' = i -+ 1 (even / odd y), clamped; columns likewise.  One thread owns a
+// 2x2 luma block (one chroma sample and its 3x3 neighbourhood): uchar2 Y loads, float2 stores of every output plane.
+__global__ void __launch_bounds__(256) yuv420p_to_rgb_lab_kernel(const uint8_t* __restrict__ yuv, float* __restrict__ rgb,
+                                                                 float* __restrict__ lab, int H, int W, YuvCoeffs k) {
+    const int Hc = H / 2, Wc = W / 2;
+    const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = blockIdx.y;
+    if (q >= (size_t)Hc * Wc) return;
+    const int i = (int)(q / Wc), j = (int)(q - (size_t)i * Wc);
+    const size_t plane = (size_t)H * W;
+    const uint8_t* Y = yuv + (size_t)n * plane * 3 / 2;
+    const uint8_t* U = Y + plane;
+    const uint8_t* V = U + plane / 4;
+    const int rows[3] = {max(i - 1, 0), i, min(i + 1, Hc - 1)}, cols[3] = {max(j - 1, 0), j, min(j + 1, Wc - 1)};
+    int u[3][3], v[3][3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b) {
+            u[a][b] = __ldg(U + (size_t)rows[a] * Wc + cols[b]);
+            v[a][b] = __ldg(V + (size_t)rows[a] * Wc + cols[b]);
+        }
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy) {
+        const size_t o = (size_t)(2 * i + dy) * W + 2 * j;
+        const uchar2 yy = __ldg(reinterpret_cast<const uchar2*>(Y + o));
+        float c[6][2];                               // r, g, b, L, a, b of the left and right pixel
+#pragma unroll
+        for (int dx = 0; dx < 2; ++dx) {
+            const int a = 2 * dy, b = 2 * dx;        // the neighbour row / column: index 0 (i - 1) or 2 (i + 1)
+            const int cb16 = 9 * u[1][1] + 3 * u[1][b] + 3 * u[a][1] + u[a][b];
+            const int cr16 = 9 * v[1][1] + 3 * v[1][b] + 3 * v[a][1] + v[a][b];
+            const uchar3 code = yuv_to_rgb_code(dx ? yy.y : yy.x, cb16, cr16, k);
+            c[0][dx] = code_value(code.x);
+            c[1][dx] = code_value(code.y);
+            c[2][dx] = code_value(code.z);
+            const float3 l = scaled_lab(c[0][dx], c[1][dx], c[2][dx]);
+            c[3][dx] = l.x;
+            c[4][dx] = l.y;
+            c[5][dx] = l.z;
+        }
+        const size_t f = (size_t)n * 3 * plane + o;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            *reinterpret_cast<float2*>(rgb + f + ch * plane) = make_float2(c[ch][0], c[ch][1]);
+            *reinterpret_cast<float2*>(lab + f + ch * plane) = make_float2(c[3 + ch][0], c[3 + ch][1]);
+        }
+    }
 }
 
 __global__ void lab2rgb_kernel(const float* __restrict__ lab, float* __restrict__ rgb, size_t plane, int B) {
@@ -443,6 +521,19 @@ extern "C" int fvfi_rgb8_to_rgb_lab(const uint8_t* rgb8, float* rgb, float* lab,
     const size_t plane = (size_t)H * W;
     dim3 grid((unsigned)((plane + 255) / 256), T);
     rgb8_to_rgb_lab_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rgb8, rgb, lab, plane);
+    FVFI_LAUNCH_CHECK();
+    return FVFI_OK;
+}
+
+extern "C" int fvfi_yuv420p_to_rgb_lab(const uint8_t* yuv, float* rgb, float* lab, int T, int H, int W, int matrix, int full_range,
+                                       void* stream) {
+    FVFI_CHECK_ARG(yuv && rgb && lab, "fvfi_yuv420p_to_rgb_lab: null pointer");
+    if (int rc = yuv_check("fvfi_yuv420p_to_rgb_lab", T, H, W, matrix, full_range)) return rc;
+    FVFI_CHECK_ARG((uintptr_t)yuv % 2 == 0 && (uintptr_t)rgb % 8 == 0 && (uintptr_t)lab % 8 == 0,
+                   "fvfi_yuv420p_to_rgb_lab: yuv must be 2-byte and rgb / lab 8-byte aligned");
+    const size_t blocks = (size_t)(H / 2) * (W / 2);
+    dim3 grid((unsigned)((blocks + 255) / 256), T);
+    yuv420p_to_rgb_lab_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(yuv, rgb, lab, H, W, yuv_coeffs(matrix, full_range));
     FVFI_LAUNCH_CHECK();
     return FVFI_OK;
 }

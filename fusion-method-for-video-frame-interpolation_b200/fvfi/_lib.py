@@ -65,6 +65,8 @@ _PROTOS = {
     "fvfi_phasenet_outputs_offset": (c_int, [c_fp, c_int, c_fp, c_fp, c_fp] + [c_int] * 8 + [c_fp]),
     "fvfi_rgb8_to_rgb_lab": (c_int, [c_fp, c_fp, c_fp, c_int, c_int, c_int, c_fp]),
     "fvfi_fusion_blend_rgb8": (c_int, [c_fp, c_fp, c_fp, c_int, c_int, c_int, c_fp]),
+    "fvfi_yuv420p_to_rgb_lab": (c_int, [c_fp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
+    "fvfi_fusion_blend_yuv420p": (c_int, [c_fp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
     "fvfi_max_pool2_nhwc": (c_int, [c_fp, c_int, c_fp, c_int, c_int, c_int, c_int, c_int, c_fp]),
     "fvfi_adacofnet_prep": (c_int, [c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_int, c_int, c_int, c_int, c_int, c_fp, c_fp]),
     "fvfi_avg_pool2_nhwc": (c_int, [c_fp, c_int, c_fp, c_int, c_int, c_int, c_int, c_int, c_fp]),

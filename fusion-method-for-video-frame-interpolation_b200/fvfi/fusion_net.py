@@ -9,7 +9,7 @@ fvfi_fusion_blend_backward (training step, SURVEY.md config 5).
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, transform
 from . import conv as tc
 
 
@@ -38,6 +38,24 @@ def fusion_blend_rgb8(base, x, out=None):
     assert out.dtype == torch.uint8 and out.shape == (B, H, W, 3) and out.is_contiguous()
     with torch.cuda.device(base.device):
         _lib.check(_lib.lib().fvfi_fusion_blend_rgb8(base.data_ptr(), x.data_ptr(), out.data_ptr(), B, H, W, _lib.stream_ptr()))
+    return out
+
+
+def fusion_blend_yuv420p(base, x, out=None, matrix="bt709", full_range=False):
+    """The yuv420p form of ``fusion_blend``: planar [B,3,H,W] in (H, W even), 8-bit planar I420 [B,3H/2,W] uint8 out (Y [H,W],
+    then U and V [H/2,W/2] per frame): Y per pixel and Cb / Cr of every 2x2 block's mean of clamp(base + tanh(x), 0, 1), with
+    ``matrix`` 'bt709' or 'bt601' and limited or ``full_range``; the fp32 frame is never stored (fvfi_fusion_blend_yuv420p)."""
+    mat, full = transform.yuv_args(matrix, full_range)
+    base = base.contiguous()
+    x = x.contiguous()
+    B, C, H, W = base.shape
+    assert C == 3 and x.shape == base.shape
+    if out is None:
+        out = torch.empty((B, 3 * H // 2, W), dtype=torch.uint8, device=base.device)
+    assert out.dtype == torch.uint8 and out.shape == (B, 3 * H // 2, W) and out.is_contiguous()
+    with torch.cuda.device(base.device):
+        _lib.check(_lib.lib().fvfi_fusion_blend_yuv420p(base.data_ptr(), x.data_ptr(), out.data_ptr(), B, H, W, mat, full,
+                                                        _lib.stream_ptr()))
     return out
 
 

@@ -1,9 +1,13 @@
-"""Frame-rate doubling of raw 8-bit video: reads rgb24 frames, writes rgb24 frames at twice the frame rate (the input frames
-with an interpolated frame between every two of them), so it sits between two ffmpeg pipes:
+"""Frame-rate doubling of raw 8-bit video: reads rgb24 or yuv420p frames, writes frames of the same format at twice the frame
+rate (the input frames with an interpolated frame between every two of them), so it sits between two ffmpeg pipes:
 
     ffmpeg -i in.mp4 -f rawvideo -pix_fmt rgb24 - \\
       | python -m fvfi.interpolate_video --size 1920x1080 --state weights.pt \\
       | ffmpeg -f rawvideo -pix_fmt rgb24 -s 1920x1080 -r 60 -i - out.mp4
+
+With ``--pix-fmt yuv420p`` (8-bit planar I420, W x H x 3/2 bytes a frame, H and W even) the decoder's frames need no conversion on
+the host, the input frames are passed through byte for byte, and ``--matrix`` (bt709 | bt601) and ``--range`` (tv | pc) say how
+the frames are converted to and from R'G'B' on the GPU.
 
 ``--state`` is a ``torch.save`` of {"phase_net", "fusion_net", "adacof"} state dicts; ``--seeded-weights SEED`` uses the
 seeded random initialisation of fvfi.synth instead (tests, benchmarks).  The clip is streamed in segments of a few windows
@@ -34,16 +38,26 @@ def _parse_size(s):
 
 def parse_args(argv=None):
     ap = argparse.ArgumentParser(prog="python -m fvfi.interpolate_video", description=__doc__.split("\n\n")[0])
-    ap.add_argument("--size", type=_parse_size, required=True, help="frame size WxH of the rgb24 stream")
+    ap.add_argument("--size", type=_parse_size, required=True, help="frame size WxH of the stream")
     ap.add_argument("--batch", type=int, default=8, help="frame pairs per window (FusionPipeline.max_batch)")
     w = ap.add_mutually_exclusive_group(required=True)
     w.add_argument("--state", help="torch.save of {'phase_net', 'fusion_net', 'adacof'} state dicts")
     w.add_argument("--seeded-weights", type=int, metavar="SEED", help="seeded random weights (fvfi.synth.seeded_state)")
-    ap.add_argument("--input", default="-", help="raw rgb24 input file, or - for stdin")
-    ap.add_argument("--output", default="-", help="raw rgb24 output file, or - for stdout")
+    ap.add_argument("--input", default="-", help="raw input file, or - for stdin")
+    ap.add_argument("--output", default="-", help="raw output file, or - for stdout")
+    ap.add_argument("--pix-fmt", choices=["rgb24", "yuv420p"], default="rgb24", help="pixel format of both streams (default rgb24)")
+    ap.add_argument("--matrix", choices=["bt709", "bt601"], help="yuv420p only: YCbCr matrix (default bt709)")
+    ap.add_argument("--range", choices=["tv", "pc"], help="yuv420p only: limited (tv, default) or full (pc) range")
     a = ap.parse_args(argv)
     if a.batch < 1:
         ap.error("--batch must be at least 1")
+    if a.pix_fmt == "yuv420p":
+        if a.size[0] % 2 or a.size[1] % 2:
+            ap.error("--pix-fmt yuv420p needs an even --size, got %dx%d" % a.size)
+        a.matrix = a.matrix or "bt709"
+        a.range = a.range or "tv"
+    elif a.matrix is not None or a.range is not None:
+        ap.error("--matrix and --range apply to --pix-fmt yuv420p only")
     return a
 
 
@@ -75,11 +89,14 @@ def _check_regular_file(f, frame_bytes):
 
 def run(args, fin, fout):
     W, H = args.size
-    frame_bytes = H * W * 3
+    yuv = args.pix_fmt == "yuv420p"
+    fshape = (H * 3 // 2, W) if yuv else (H, W, 3)     # one frame: I420 planes [3H/2,W] or interleaved rgb24 [H,W,3]
+    frame_bytes = H * W * 3 // 2 if yuv else H * W * 3
+    fmt = dict(pix_fmt="yuv420p", matrix=args.matrix, full_range=args.range == "pc") if yuv else {}
     _check_regular_file(fin, frame_bytes)
     seg = args.batch * WINDOWS_PER_SEGMENT             # pairs per segment
     import numpy as np
-    head = np.empty((2, H, W, 3), dtype=np.uint8)      # the first two frames decide "at least 2 frames" before CUDA is touched
+    head = np.empty((2,) + fshape, dtype=np.uint8)     # the first two frames decide "at least 2 frames" before CUDA is touched
     n = _read_into(fin, memoryview(head).cast("B"))
     if n < 2 * frame_bytes:
         if n % frame_bytes:
@@ -94,8 +111,8 @@ def run(args, fin, fout):
     pipe = FusionPipeline(H, W, "cuda")
     pipe.load_state(state)
     pipe.max_batch = args.batch
-    frames = torch.empty((seg + 1, H, W, 3), dtype=torch.uint8).pin_memory()
-    out = torch.empty((2 * seg + 1, H, W, 3), dtype=torch.uint8).pin_memory()
+    frames = torch.empty((seg + 1,) + fshape, dtype=torch.uint8).pin_memory()
+    out = torch.empty((2 * seg + 1,) + fshape, dtype=torch.uint8).pin_memory()
     fbytes = memoryview(frames.numpy()).cast("B")
     frames.numpy()[:2] = head
     have, first = 2, True                              # frames in the buffer; after a segment, frame 0 is its last frame
@@ -106,7 +123,7 @@ def run(args, fin, fout):
         have += got // frame_bytes
         eof = have < seg + 1                           # the buffer was not filled: the stream has ended
         if have >= 2:
-            pipe.interpolate_video_host(frames[:have], out[:2 * have - 1])
+            pipe.interpolate_video_host(frames[:have], out[:2 * have - 1], **fmt)
             fout.write(memoryview(out.numpy()[0 if first else 1:2 * have - 1]).cast("B"))
             first = False
             frames[0].copy_(frames[have - 1])          # the boundary frame starts the next segment

@@ -17,7 +17,7 @@ import torch
 from . import conv as tc
 from . import filters, transform, utils
 from .adacofnet import AdaCoFNet
-from .fusion_net import FusionNet, fusion_blend_rgb8
+from .fusion_net import FusionNet, fusion_blend_rgb8, fusion_blend_yuv420p
 from .phase_net import PhaseNet
 from .pyramid import Pyramid
 
@@ -258,36 +258,57 @@ class FusionPipeline(torch.nn.Module):
                 self.stages["phase%d" % l], self.stages["amp%d" % l] = p, a
         return phase_pred
 
-    def _check_clip(self, frames):
-        """Validates a clip for interpolate_sequence; returns True for 8-bit [T,H,W,3], False for fp32 [T,3,H,W]."""
-        if not torch.is_tensor(frames) or frames.dim() != 4:
-            raise ValueError("a clip is a 4-d tensor: float32 [T,3,H,W] or uint8 [T,H,W,3]")
-        if frames.dtype == torch.uint8:
-            shape, want = tuple(frames.shape[1:]), (self.H, self.W, 3)
-        elif frames.dtype == torch.float32:
-            shape, want = tuple(frames.shape[1:]), (3, self.H, self.W)
+    def _check_clip(self, frames, pix_fmt=None, matrix="bt709", full_range=False):
+        """Validates a clip for interpolate_sequence; returns True for 8-bit frames (rgb24 [T,H,W,3] or, with pix_fmt='yuv420p',
+        [T,3H/2,W]), False for fp32 [T,3,H,W]."""
+        if pix_fmt == "yuv420p":
+            transform.yuv_args(matrix, full_range)
+            if self.H % 2 or self.W % 2:
+                raise ValueError("yuv420p needs an even frame size; this pipeline is %dx%d" % (self.W, self.H))
+            want = (3 * self.H // 2, self.W)
+            if not torch.is_tensor(frames) or frames.dim() != 3 or frames.dtype != torch.uint8:
+                raise ValueError("a yuv420p clip is a uint8 tensor [T,3H/2,W] = [T,%d,%d] for this pipeline" % want)
+            if tuple(frames.shape[1:]) != want:
+                raise ValueError("yuv420p clip frames must be %s for this %dx%d pipeline, got %s"
+                                 % (list(want), self.W, self.H, list(frames.shape[1:])))
+        elif pix_fmt is not None:
+            raise ValueError("pix_fmt must be None (the dtype and layout decide) or 'yuv420p', got %r" % (pix_fmt,))
         else:
-            raise ValueError("clip dtype must be torch.float32 ([T,3,H,W] in [0,1]) or torch.uint8 ([T,H,W,3]), got %s" % frames.dtype)
-        if shape != want:
-            raise ValueError("%s clip frames must be %s for this %dx%d pipeline, got %s (wrong frame size or layout)"
-                             % (frames.dtype, list(want), self.W, self.H, list(shape)))
+            if not torch.is_tensor(frames) or frames.dim() != 4:
+                raise ValueError("a clip is a 4-d tensor: float32 [T,3,H,W] or uint8 [T,H,W,3]")
+            if frames.dtype == torch.uint8:
+                shape, want = tuple(frames.shape[1:]), (self.H, self.W, 3)
+            elif frames.dtype == torch.float32:
+                shape, want = tuple(frames.shape[1:]), (3, self.H, self.W)
+            else:
+                raise ValueError("clip dtype must be torch.float32 ([T,3,H,W] in [0,1]) or torch.uint8 ([T,H,W,3]), got %s"
+                                 % frames.dtype)
+            if shape != want:
+                raise ValueError("%s clip frames must be %s for this %dx%d pipeline, got %s (wrong frame size or layout)"
+                                 % (frames.dtype, list(want), self.W, self.H, list(shape)))
         if frames.shape[0] < 2:
             raise ValueError("a clip needs at least 2 frames, got %d" % frames.shape[0])
         return frames.dtype == torch.uint8
 
-    def _clip_window(self, frames, out=None):
+    def _clip_window(self, frames, out=None, pix_fmt=None, matrix="bt709", full_range=False):
         """Interpolates the B pairs of a window of B + 1 consecutive frames (device tensors in interpolate_sequence's formats):
         Lab and the pyramid decomposition run once per frame, the pairs read them as views (clip layout, q = 3).  Writes the B new
-        frames into ``out`` (allocated if None) in the input's dtype and layout."""
+        frames into ``out`` (allocated if None) in the input's format."""
         H, W = self.H, self.W
+        yuv = pix_fmt == "yuv420p"
         self._tick('start')
-        if frames.dtype == torch.uint8:
+        if yuv:
+            rgb, lab = transform.yuv420p_to_rgb_lab(frames, matrix, full_range)
+        elif frames.dtype == torch.uint8:
             rgb, lab = transform.rgb8_to_rgb_lab(frames)
         else:
             rgb = frames.contiguous()
             lab = transform.rgb2lab(rgb)
         base, ada_pred, phase_pred, other, maps = self._fusion_inputs(rgb[:-1], rgb[1:], lab[:-1], lab[1:], lab.reshape(-1, H, W), 3)
-        if frames.dtype == torch.uint8:
+        if yuv:
+            x = self.fusion_net.residual(base, ada_pred, phase_pred, other, maps)
+            out = fusion_blend_yuv420p(base, x, out, matrix, full_range)
+        elif frames.dtype == torch.uint8:
             x = self.fusion_net.residual(base, ada_pred, phase_pred, other, maps)
             out = fusion_blend_rgb8(base, x, out)
         else:
@@ -298,37 +319,42 @@ class FusionPipeline(torch.nn.Module):
 
     @torch.no_grad()
     @tc.range_checked
-    def interpolate_sequence(self, frames):
+    def interpolate_sequence(self, frames, pix_fmt=None, matrix="bt709", full_range=False):
         """The T - 1 in-between frames of a clip on the device: fp32 [T,3,H,W] in [0,1] -> fp32 [T-1,3,H,W], or uint8 [T,H,W,3]
-        (rgb24) -> uint8 [T-1,H,W,3] (8-bit in and out: no fp32 frame is stored at either end).  Frame t of the result lies
-        between input frames t and t + 1.  Works in windows of ``max_batch`` pairs; a window of B pairs converts and decomposes
-        its B + 1 frames once (the pair form ``pipe(frames[:-1], frames[1:])`` does every interior frame twice); the frame
-        between two windows is done again in the next one.  ValueError for fewer than 2 frames, a wrong frame size, dtype or
-        layout."""
-        u8 = self._check_clip(frames)
+        (rgb24) -> uint8 [T-1,H,W,3] (8-bit in and out: no fp32 frame is stored at either end).  With ``pix_fmt='yuv420p'`` the
+        clip is 8-bit planar I420, uint8 [T,3H/2,W] -> [T-1,3H/2,W] (H, W even), converted with ``matrix`` ('bt709' or 'bt601')
+        and limited or ``full_range`` at both ends (transform.yuv420p_to_rgb_lab, fusion_net.fusion_blend_yuv420p).  Frame t of
+        the result lies between input frames t and t + 1.  Works in windows of ``max_batch`` pairs; a window of B pairs converts
+        and decomposes its B + 1 frames once (the pair form ``pipe(frames[:-1], frames[1:])`` does every interior frame twice);
+        the frame between two windows is done again in the next one.  ValueError for fewer than 2 frames, a wrong frame size,
+        dtype or layout."""
+        u8 = self._check_clip(frames, pix_fmt, matrix, full_range)
         if not frames.is_cuda:
             raise ValueError("interpolate_sequence takes device tensors (interpolate_video_host takes host frames)")
         T, mb = frames.shape[0], self.max_batch
         out = torch.empty((T - 1,) + tuple(frames.shape[1:]), dtype=torch.uint8 if u8 else torch.float32, device=frames.device)
         for a in range(0, T - 1, mb):
             b = min(mb, T - 1 - a)
-            self._clip_window(frames[a:a + b + 1], out[a:a + b])
+            self._clip_window(frames[a:a + b + 1], out[a:a + b], pix_fmt, matrix, full_range)
         return out
 
-    def interpolate_video_host(self, frames_host, out_host=None):
-        """Clip on HOST (pinned) memory: uint8 [T,H,W,3] rgb24 -> uint8 [2T-1,H,W,3], the input frames at even indices and the
-        interpolated ones at odd indices (twice the frame rate).  Windows of ``max_batch`` pairs go up as 8-bit frames and come
-        back as 8-bit frames on the two copy streams of interpolate_host, overlapped with the compute of the neighbouring
-        windows; the input frames are copied into the even slots on the host meanwhile."""
+    def interpolate_video_host(self, frames_host, out_host=None, pix_fmt=None, matrix="bt709", full_range=False):
+        """Clip on HOST (pinned) memory: uint8 [T,H,W,3] rgb24 -> uint8 [2T-1,H,W,3], or with ``pix_fmt='yuv420p'`` uint8
+        [T,3H/2,W] -> [2T-1,3H/2,W] (``matrix``, ``full_range`` as interpolate_sequence), the input frames at even indices and
+        the interpolated ones at odd indices (twice the frame rate).  Windows of ``max_batch`` pairs go up as 8-bit frames and
+        come back as 8-bit frames on the two copy streams of interpolate_host, overlapped with the compute of the neighbouring
+        windows; the input frames are copied into the even slots on the host meanwhile, byte for byte."""
+        layout = "[T,3H/2,W] yuv420p" if pix_fmt == "yuv420p" else "[T,H,W,3]"
         if not torch.is_tensor(frames_host) or frames_host.is_cuda or frames_host.dtype != torch.uint8:
-            raise ValueError("interpolate_video_host takes a host uint8 [T,H,W,3] tensor (pinned for overlapped copies)")
-        self._check_clip(frames_host)
+            raise ValueError("interpolate_video_host takes a host uint8 %s tensor (pinned for overlapped copies)" % layout)
+        self._check_clip(frames_host, pix_fmt, matrix, full_range)
         frames_host = frames_host.contiguous()
-        T, H, W = frames_host.shape[0], self.H, self.W
+        T = frames_host.shape[0]
+        shape = (2 * T - 1,) + tuple(frames_host.shape[1:])
         if out_host is None:
-            out_host = torch.empty((2 * T - 1, H, W, 3), dtype=torch.uint8).pin_memory()
-        if tuple(out_host.shape) != (2 * T - 1, H, W, 3) or out_host.dtype != torch.uint8 or out_host.is_cuda:
-            raise ValueError("out_host must be a host uint8 [%d,%d,%d,3] tensor" % (2 * T - 1, H, W))
+            out_host = torch.empty(shape, dtype=torch.uint8).pin_memory()
+        if tuple(out_host.shape) != shape or out_host.dtype != torch.uint8 or out_host.is_cuda:
+            raise ValueError("out_host must be a host uint8 [%s] tensor" % ",".join(map(str, shape)))
         mb = self.max_batch
         starts = list(range(0, T - 1, mb))
         uploads = [(frames_host[a:a + min(mb, T - 1 - a) + 1],) for a in starts]
@@ -339,7 +365,7 @@ class FusionPipeline(torch.nn.Module):
 
         def host_work():
             out_host[0::2].copy_(frames_host)
-        self._run_windows(uploads, self._clip_window, download, host_work)
+        self._run_windows(uploads, lambda frames: self._clip_window(frames, None, pix_fmt, matrix, full_range), download, host_work)
         return out_host
 
     def interpolate_host(self, rgb1_host, rgb2_host, out_host=None):

@@ -51,6 +51,48 @@ def rgb8_to_rgb_lab(frames8):
     return rgb, lab
 
 
+YUV_MATRICES = {"bt709": 709, "bt601": 601}
+
+
+def yuv_args(matrix, full_range):
+    """The (matrix, full_range) integers of the yuv420p entry points: 'bt709' -> 709, 'bt601' -> 601; limited (tv) range -> 0,
+    full (pc) range -> 1.  ValueError for anything else."""
+    if matrix not in YUV_MATRICES:
+        raise ValueError("matrix must be one of %s, got %r" % (sorted(YUV_MATRICES), matrix))
+    if full_range not in (False, True):
+        raise ValueError("full_range must be a bool, got %r" % (full_range,))
+    return YUV_MATRICES[matrix], int(full_range)
+
+
+def yuv420p_frame_size(frames):
+    """(H, W) of a yuv420p clip [T,3H/2,W] uint8 (ValueError if it is not one)."""
+    if not torch.is_tensor(frames) or frames.dtype != torch.uint8 or frames.dim() != 3:
+        raise ValueError("a yuv420p clip is a uint8 tensor [T,3H/2,W]")
+    rows, W = frames.shape[1:]
+    if rows % 3 or W % 2:
+        raise ValueError("yuv420p frames [3H/2,W] need an even H and W, got [%d,%d]" % (rows, W))
+    return 2 * rows // 3, W
+
+
+def yuv420p_to_rgb_lab(frames, matrix="bt709", full_range=False):
+    """Decoder frames [T,3H/2,W] uint8, 8-bit planar I420 as ffmpeg's ``-pix_fmt yuv420p`` writes them (Y [H,W], then U and V
+    [H/2,W/2], contiguous per frame) -> (rgb, lab), planar fp32 [T,3,H,W], in one kernel (fvfi_yuv420p_to_rgb_lab).  ``rgb`` is
+    the correctly rounded k / 255 of the rgb24 frame this conversion gives (centre-sited chroma upsampled bilinearly, ``matrix``
+    'bt709' or 'bt601', limited or ``full_range``); ``lab`` equals ``rgb2lab(rgb)`` bit for bit."""
+    if not frames.is_cuda:
+        raise NotImplementedError("fvfi colour transforms run on CUDA tensors only")
+    mat, full = yuv_args(matrix, full_range)
+    H, W = yuv420p_frame_size(frames)
+    x = frames.contiguous()
+    T = x.shape[0]
+    rgb = torch.empty((T, 3, H, W), dtype=torch.float32, device=x.device)
+    lab = torch.empty_like(rgb)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().fvfi_yuv420p_to_rgb_lab(x.data_ptr(), rgb.data_ptr(), lab.data_ptr(), T, H, W, mat, full,
+                                                      _lib.stream_ptr()))
+    return rgb, lab
+
+
 def lab2rgb_single(img, light=100, ab_mul=255, ab_max=128):
     """[3,H,W] (transform.py:40-49)."""
     return lab2rgb(img.unsqueeze(0), light, ab_mul, ab_max)[0]

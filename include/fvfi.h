@@ -104,6 +104,14 @@ int fvfi_fusion_blend(const float* base, const float* x_pre_tanh, float* out, si
 /* The same blend for 8-bit output: base / x_pre_tanh [B,3,H,W] planar -> out [B,H,W,3] uint8 interleaved (rgb24),
  * out = rint(clamp(base + tanh(x), 0, 1) * 255) with ties to even.  The fp32 frame is never written. */
 int fvfi_fusion_blend_rgb8(const float* base, const float* x_pre_tanh, uint8_t* out, int B, int H, int W, void* stream);
+/* The same blend for yuv420p output: base / x_pre_tanh [B,3,H,W] planar -> out [B,3H/2,W] uint8, 8-bit planar I420 (Y [H,W], then
+ * U [H/2,W/2], then V [H/2,W/2] per frame, contiguous; ffmpeg -pix_fmt yuv420p).  For R, G, B = clamp(base + tanh(x), 0, 1):
+ * Y = rint(yoff + ys ((Kr R + Kg G) + Kb B)) per pixel; Cb = rint(128 + cs ((Bm - Ym) / (2(1 - Kb)))) and Cr likewise from the 2x2
+ * block means Rm = ((R00 + R01) + (R10 + R11)) / 4 (centre-sited chroma), Ym their luma; every value clamped to [0, 255], ties to
+ * even, every product and sum rounded separately.  matrix: 709 or 601; full_range: 0 = limited (16, 219, 224), 1 = full (0, 255,
+ * 255).  H and W even, B <= 65535, base / x_pre_tanh 8-byte and out 2-byte aligned.  The fp32 frame is never written. */
+int fvfi_fusion_blend_yuv420p(const float* base, const float* x_pre_tanh, uint8_t* out, int B, int H, int W, int matrix,
+                              int full_range, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Per-pixel stages the reference runs on the host CPU (SURVEY.md 8(f) f1/f2), device-resident here.
@@ -114,6 +122,15 @@ int fvfi_lab2rgb(const float* lab, float* rgb, int B, int H, int W, void* stream
 /* Decoder frames rgb8 [T,H,W,3] uint8 interleaved (ffmpeg -pix_fmt rgb24) -> rgb [T,3,H,W] planar fp32 (the correctly rounded
  * k / 255) and lab [T,3,H,W] planar scaled Lab, in one pass; lab is bit-identical to fvfi_rgb2lab of rgb. */
 int fvfi_rgb8_to_rgb_lab(const uint8_t* rgb8, float* rgb, float* lab, int T, int H, int W, void* stream);
+/* Decoder frames yuv [T,3H/2,W] uint8, 8-bit planar I420 (ffmpeg -pix_fmt yuv420p, layout as fvfi_fusion_blend_yuv420p) -> rgb and
+ * lab [T,3,H,W] as fvfi_rgb8_to_rgb_lab gives them for the rgb24 frame of this conversion: centre-sited chroma upsampled by the
+ * [1,3]/4 bilinear filter in each direction (cb16 = 9 U[i][j] + 3 U[i][j'] + 3 U[i'][j] + U[i'][j'], i = y/2, i' = i - 1 for even y
+ * and i + 1 for odd y, clamped; j' likewise), Y' = (Y - yoff) / ys, Cb' = (cb16 - 2048) / (16 cs), R = Y' + 2(1 - Kr) Cr',
+ * B = Y' + 2(1 - Kb) Cb', G = (Y' - 2Kb(1 - Kb)/Kg Cb') - 2Kr(1 - Kr)/Kg Cr', code = rint(clamp(v, 0, 1) * 255), every operation
+ * rounded separately.  No transfer or primaries conversion: the codes are used as sRGB values, as rgb24 input is.  matrix: 709 or
+ * 601; full_range: 0 = limited, 1 = full; H and W even, T <= 65535, yuv 2-byte and rgb / lab 8-byte aligned. */
+int fvfi_yuv420p_to_rgb_lab(const uint8_t* yuv, float* rgb, float* lab, int T, int H, int W, int matrix, int full_range,
+                            void* stream);
 /* scipy.ndimage.gaussian_filter(x, sigma) on N maps [N,H,W] (truncate 4, mode 'reflect';
  * src/fusion_net/interpolate_twoframe.py:212-213).  tmp: scratch of the same size. */
 int fvfi_gaussian_filter(const float* in, float* out, float* tmp, int N, int H, int W, float sigma, void* stream);
