@@ -67,6 +67,9 @@ _PROTOS = {
     "fvfi_fusion_blend_rgb8": (c_int, [c_fp, c_fp, c_fp, c_int, c_int, c_int, c_fp]),
     "fvfi_yuv420p_to_rgb_lab": (c_int, [c_fp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
     "fvfi_fusion_blend_yuv420p": (c_int, [c_fp, c_fp, c_fp] + [c_int] * 5 + [c_fp]),
+    "fvfi_frame_sad_u8": (c_int, [c_fp, c_size, c_size, c_int, c_fp, c_fp]),
+    "fvfi_scene_cut_decide": (c_int, [c_fp, c_int, c_size, c_fp, ctypes.c_double, c_fp, c_fp, c_fp]),
+    "fvfi_scene_cut_select_u8": (c_int, [c_fp, c_size, c_fp, c_size, c_size, c_int, c_fp, c_fp]),
     "fvfi_max_pool2_nhwc": (c_int, [c_fp, c_int, c_fp, c_int, c_int, c_int, c_int, c_int, c_fp]),
     "fvfi_adacofnet_prep": (c_int, [c_fp, c_fp, c_fp, c_fp, c_fp, c_int, c_int, c_int, c_int, c_int, c_int, c_fp, c_fp]),
     "fvfi_avg_pool2_nhwc": (c_int, [c_fp, c_int, c_fp, c_int, c_int, c_int, c_int, c_int, c_fp]),

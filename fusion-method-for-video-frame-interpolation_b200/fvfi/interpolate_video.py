@@ -9,6 +9,10 @@ With ``--pix-fmt yuv420p`` (8-bit planar I420, W x H x 3/2 bytes a frame, H and 
 the host, the input frames are passed through byte for byte, and ``--matrix`` (bt709 | bt601) and ``--range`` (tv | pc) say how
 the frames are converted to and from R'G'B' on the GPU.
 
+``--scene-threshold T`` turns scene-cut detection on (fvfi.scene; off by default): at a cut the earlier frame is repeated instead of
+an interpolated frame, and ``--scene-log PATH`` lists the pair index of every cut (pair p lies between input frames p and p + 1),
+one per line.  One detector serves the whole stream, so the result does not depend on ``--batch``.
+
 ``--state`` is a ``torch.save`` of {"phase_net", "fusion_net", "adacof"} state dicts; ``--seeded-weights SEED`` uses the
 seeded random initialisation of fvfi.synth instead (tests, benchmarks).  The clip is streamed in segments of a few windows
 of ``--batch`` pairs, so host and device memory stay bounded for any length.  A regular input file whose size is not a
@@ -16,6 +20,7 @@ whole number of frames, or that holds fewer than 2 frames, is rejected before an
 are rejected the same way and a partial last frame is an error when the stream ends.
 """
 import argparse
+import math
 import os
 import sys
 
@@ -36,6 +41,16 @@ def _parse_size(s):
     return w, h
 
 
+def _parse_threshold(s):
+    try:
+        t = float(s)
+    except ValueError:
+        t = math.nan
+    if not math.isfinite(t) or t < 0:
+        raise argparse.ArgumentTypeError("--scene-threshold must be a finite number >= 0, got %r" % s)
+    return t
+
+
 def parse_args(argv=None):
     ap = argparse.ArgumentParser(prog="python -m fvfi.interpolate_video", description=__doc__.split("\n\n")[0])
     ap.add_argument("--size", type=_parse_size, required=True, help="frame size WxH of the stream")
@@ -48,6 +63,9 @@ def parse_args(argv=None):
     ap.add_argument("--pix-fmt", choices=["rgb24", "yuv420p"], default="rgb24", help="pixel format of both streams (default rgb24)")
     ap.add_argument("--matrix", choices=["bt709", "bt601"], help="yuv420p only: YCbCr matrix (default bt709)")
     ap.add_argument("--range", choices=["tv", "pc"], help="yuv420p only: limited (tv, default) or full (pc) range")
+    ap.add_argument("--scene-threshold", type=_parse_threshold, metavar="T",
+                    help="repeat the earlier frame at scene cuts with a score >= T (0-100, ~10 as ffmpeg's scd_threshold; default off)")
+    ap.add_argument("--scene-log", metavar="PATH", help="with --scene-threshold: write the pair index of every cut, one per line")
     a = ap.parse_args(argv)
     if a.batch < 1:
         ap.error("--batch must be at least 1")
@@ -58,6 +76,8 @@ def parse_args(argv=None):
         a.range = a.range or "tv"
     elif a.matrix is not None or a.range is not None:
         ap.error("--matrix and --range apply to --pix-fmt yuv420p only")
+    if a.scene_log is not None and a.scene_threshold is None:
+        ap.error("--scene-log needs --scene-threshold")
     return a
 
 
@@ -111,6 +131,11 @@ def run(args, fin, fout):
     pipe = FusionPipeline(H, W, "cuda")
     pipe.load_state(state)
     pipe.max_batch = args.batch
+    scene = None
+    if args.scene_threshold is not None:
+        from .scene import SceneCutDetector
+        scene = SceneCutDetector(args.scene_threshold)     # one detector for the stream: its carry crosses the segments
+        fmt["scene_cut"] = scene
     frames = torch.empty((seg + 1,) + fshape, dtype=torch.uint8).pin_memory()
     out = torch.empty((2 * seg + 1,) + fshape, dtype=torch.uint8).pin_memory()
     fbytes = memoryview(frames.numpy()).cast("B")
@@ -131,6 +156,9 @@ def run(args, fin, fout):
         if eof:
             break
     fout.flush()
+    if args.scene_log is not None:
+        with open(args.scene_log, "w") as log:
+            log.writelines("%d\n" % p for p in scene.cuts)
 
 
 def main(argv=None):

@@ -20,6 +20,7 @@ from .adacofnet import AdaCoFNet
 from .fusion_net import FusionNet, fusion_blend_rgb8, fusion_blend_yuv420p
 from .phase_net import PhaseNet
 from .pyramid import Pyramid
+from .scene import SceneCutDetector
 
 
 class GraphedCall:
@@ -290,13 +291,29 @@ class FusionPipeline(torch.nn.Module):
             raise ValueError("a clip needs at least 2 frames, got %d" % frames.shape[0])
         return frames.dtype == torch.uint8
 
-    def _clip_window(self, frames, out=None, pix_fmt=None, matrix="bt709", full_range=False):
+    def _scene_call(self, scene_cut, u8, frames, pix_fmt):
+        """The per-call state of a SceneCutDetector for a clip that passed _check_clip (None without a detector)."""
+        if scene_cut is None:
+            return None
+        if not isinstance(scene_cut, SceneCutDetector):
+            raise ValueError("scene_cut must be a fvfi.scene.SceneCutDetector or None, got %r" % (scene_cut,))
+        if not u8:
+            raise ValueError("scene-cut detection takes 8-bit clips (rgb24 or yuv420p), not float32 ones")
+        n = self.H * self.W * (1 if pix_fmt == "yuv420p" else 3)     # yuv420p: the Y plane; rgb24: every byte
+        return scene_cut.begin(frames.shape[0] - 1, n, self.device)
+
+    def _clip_window(self, frames, out=None, pix_fmt=None, matrix="bt709", full_range=False, scene=None, a=0):
         """Interpolates the B pairs of a window of B + 1 consecutive frames (device tensors in interpolate_sequence's formats):
         Lab and the pyramid decomposition run once per frame, the pairs read them as views (clip layout, q = 3).  Writes the B new
-        frames into ``out`` (allocated if None) in the input's format."""
+        frames into ``out`` (allocated if None) in the input's format.  ``scene`` (a fvfi.scene.SceneCall; 8-bit clips): the
+        window's pairs are pairs a .. a + B - 1 of the call; at a detected cut the new frame is replaced by the earlier input
+        frame, on this stream, before the caller's download."""
         H, W = self.H, self.W
         yuv = pix_fmt == "yuv420p"
         self._tick('start')
+        if scene is not None:
+            frames = frames.contiguous()
+            scene.detect(frames, a)
         if yuv:
             rgb, lab = transform.yuv420p_to_rgb_lab(frames, matrix, full_range)
         elif frames.dtype == torch.uint8:
@@ -314,40 +331,54 @@ class FusionPipeline(torch.nn.Module):
         else:
             final = self.fusion_net(base, ada_pred, phase_pred, other, maps, variant=0)
             out = final if out is None else out.copy_(final)
+        if scene is not None:
+            scene.select(frames, out, a)
         self._tick('fusion_net')
         return out
 
     @torch.no_grad()
-    @tc.range_checked
-    def interpolate_sequence(self, frames, pix_fmt=None, matrix="bt709", full_range=False):
+    def interpolate_sequence(self, frames, pix_fmt=None, matrix="bt709", full_range=False, scene_cut=None):
         """The T - 1 in-between frames of a clip on the device: fp32 [T,3,H,W] in [0,1] -> fp32 [T-1,3,H,W], or uint8 [T,H,W,3]
         (rgb24) -> uint8 [T-1,H,W,3] (8-bit in and out: no fp32 frame is stored at either end).  With ``pix_fmt='yuv420p'`` the
         clip is 8-bit planar I420, uint8 [T,3H/2,W] -> [T-1,3H/2,W] (H, W even), converted with ``matrix`` ('bt709' or 'bt601')
         and limited or ``full_range`` at both ends (transform.yuv420p_to_rgb_lab, fusion_net.fusion_blend_yuv420p).  Frame t of
         the result lies between input frames t and t + 1.  Works in windows of ``max_batch`` pairs; a window of B pairs converts
         and decomposes its B + 1 frames once (the pair form ``pipe(frames[:-1], frames[1:])`` does every interior frame twice);
-        the frame between two windows is done again in the next one.  ValueError for fewer than 2 frames, a wrong frame size,
-        dtype or layout."""
+        the frame between two windows is done again in the next one.  ``scene_cut`` (a fvfi.scene.SceneCutDetector, 8-bit clips
+        only): result frame t is input frame t, byte for byte, wherever pair t is a scene cut; the detector's carry and cut list
+        advance by this call.  ValueError for fewer than 2 frames, a wrong frame size, dtype or layout, or a detector with a
+        float32 clip."""
         u8 = self._check_clip(frames, pix_fmt, matrix, full_range)
         if not frames.is_cuda:
             raise ValueError("interpolate_sequence takes device tensors (interpolate_video_host takes host frames)")
+        scene = self._scene_call(scene_cut, u8, frames, pix_fmt)
+        out = self._sequence_windows(frames, u8, pix_fmt, matrix, full_range, scene)
+        if scene is not None:
+            scene.commit()          # once, after the range guard's possible second run
+        return out
+
+    @tc.range_checked
+    def _sequence_windows(self, frames, u8, pix_fmt, matrix, full_range, scene):
         T, mb = frames.shape[0], self.max_batch
         out = torch.empty((T - 1,) + tuple(frames.shape[1:]), dtype=torch.uint8 if u8 else torch.float32, device=frames.device)
         for a in range(0, T - 1, mb):
             b = min(mb, T - 1 - a)
-            self._clip_window(frames[a:a + b + 1], out[a:a + b], pix_fmt, matrix, full_range)
+            self._clip_window(frames[a:a + b + 1], out[a:a + b], pix_fmt, matrix, full_range, scene, a)
         return out
 
-    def interpolate_video_host(self, frames_host, out_host=None, pix_fmt=None, matrix="bt709", full_range=False):
+    def interpolate_video_host(self, frames_host, out_host=None, pix_fmt=None, matrix="bt709", full_range=False, scene_cut=None):
         """Clip on HOST (pinned) memory: uint8 [T,H,W,3] rgb24 -> uint8 [2T-1,H,W,3], or with ``pix_fmt='yuv420p'`` uint8
         [T,3H/2,W] -> [2T-1,3H/2,W] (``matrix``, ``full_range`` as interpolate_sequence), the input frames at even indices and
         the interpolated ones at odd indices (twice the frame rate).  Windows of ``max_batch`` pairs go up as 8-bit frames and
         come back as 8-bit frames on the two copy streams of interpolate_host, overlapped with the compute of the neighbouring
-        windows; the input frames are copied into the even slots on the host meanwhile, byte for byte."""
+        windows; the input frames are copied into the even slots on the host meanwhile, byte for byte.  ``scene_cut`` (a
+        fvfi.scene.SceneCutDetector): at a detected cut t, odd slot 2t + 1 equals even slot 2t (the earlier frame is repeated);
+        the decision and the substitution run on the device before each window's download."""
         layout = "[T,3H/2,W] yuv420p" if pix_fmt == "yuv420p" else "[T,H,W,3]"
         if not torch.is_tensor(frames_host) or frames_host.is_cuda or frames_host.dtype != torch.uint8:
             raise ValueError("interpolate_video_host takes a host uint8 %s tensor (pinned for overlapped copies)" % layout)
         self._check_clip(frames_host, pix_fmt, matrix, full_range)
+        scene = self._scene_call(scene_cut, True, frames_host, pix_fmt)
         frames_host = frames_host.contiguous()
         T = frames_host.shape[0]
         shape = (2 * T - 1,) + tuple(frames_host.shape[1:])
@@ -365,7 +396,10 @@ class FusionPipeline(torch.nn.Module):
 
         def host_work():
             out_host[0::2].copy_(frames_host)
-        self._run_windows(uploads, lambda frames: self._clip_window(frames, None, pix_fmt, matrix, full_range), download, host_work)
+        self._run_windows(uploads, lambda k, frames: self._clip_window(frames, None, pix_fmt, matrix, full_range, scene, starts[k]),
+                          download, host_work)
+        if scene is not None:
+            scene.commit()          # once, after the range guard's possible second run
         return out_host
 
     def interpolate_host(self, rgb1_host, rgb2_host, out_host=None):
@@ -380,14 +414,14 @@ class FusionPipeline(torch.nn.Module):
 
         def download(k, out):
             out_host[starts[k]:starts[k] + out.shape[0]].copy_(out, non_blocking=True)
-        self._run_windows(uploads, self.forward, download)
+        self._run_windows(uploads, lambda k, rgb1, rgb2: self.forward(rgb1, rgb2), download)
         return out_host
 
     @torch.no_grad()
     @tc.range_checked       # ONE range check (stream sync) for the whole call; the per-window calls below are nested in it
     def _run_windows(self, uploads, run, download, host_work=None):
         """Stream choreography of the host-buffer entry points: ``uploads`` [k] is the tuple of host tensors of window k; their
-        host -> device copies are all queued at once on the input stream (in order), window k's ``run(*device_tensors)`` waits for
+        host -> device copies are all queued at once on the input stream (in order), window k's ``run(k, *device_tensors)`` waits for
         its own copies only, and ``download(k, result)`` issues its device -> host copies on the output stream after the window's
         compute.  ``host_work()`` (optional) runs on the host while the device works; the call returns with every result on the
         host."""
@@ -407,7 +441,7 @@ class FusionPipeline(torch.nn.Module):
             compute.wait_event(ev)
             for d in ds:
                 d.record_stream(compute)
-            out = run(*ds)
+            out = run(k, *ds)
             done = torch.cuda.Event()
             done.record(compute)
             with torch.cuda.stream(s_out):

@@ -131,6 +131,23 @@ int fvfi_rgb8_to_rgb_lab(const uint8_t* rgb8, float* rgb, float* lab, int T, int
  * 601; full_range: 0 = limited, 1 = full; H and W even, T <= 65535, yuv 2-byte and rgb / lab 8-byte aligned. */
 int fvfi_yuv420p_to_rgb_lab(const uint8_t* yuv, float* rgb, float* lab, int T, int H, int W, int matrix, int full_range,
                             void* stream);
+
+/* Scene-cut detection on 8-bit clips (DESIGN.md 6b; oracle/scene.py restates the rule in numpy).  A window holds pairs + 1 frames,
+ * stride bytes apart; pair p = frames p and p + 1.  The compared bytes are the first n of each frame: the Y plane (n = H W) of
+ * yuv420p, all 3 H W bytes of rgb24.  All three take 1 <= pairs <= 65535 and reject bad arguments with FVFI_EINVAL before any CUDA call.
+ *   fvfi_frame_sad_u8: sad[p] = sum_i |f[p+1][i] - f[p][i]| over the n bytes, exact 64-bit integers; sad is zeroed by the call.  Each
+ *     frame byte is read once; 0 < n <= stride (16-byte loads when frames and stride are 16-byte aligned, byte loads otherwise).
+ *   fvfi_scene_cut_decide: mafd[p] = sad[p] * 100 / n / 256 in double, each operation rounded to nearest on its own;
+ *     score = clamp(min(mafd[p], |mafd[p] - prev|), 0, 100) with prev = mafd[p - 1], and for p = 0 *prev_in (the last mafd of the
+ *     stream's previous window), or 0 if prev_in is NULL (start of a stream); cut[p] = score >= threshold (0 / 1).  threshold >= 0,
+ *     not NaN.
+ *   fvfi_scene_cut_select_u8: out[p] (out_stride bytes apart) = the frame_bytes bytes of frame p where cut[p] != 0: at a cut the
+ *     earlier frame is repeated instead of an interpolated one.  Other outputs are not touched.  frame_bytes <= stride, out_stride. */
+int fvfi_frame_sad_u8(const uint8_t* frames, size_t stride, size_t n, int pairs, unsigned long long* sad, void* stream);
+int fvfi_scene_cut_decide(const unsigned long long* sad, int pairs, size_t n, const double* prev_in, double threshold, double* mafd,
+                          uint8_t* cut, void* stream);
+int fvfi_scene_cut_select_u8(const uint8_t* frames, size_t stride, uint8_t* out, size_t out_stride, size_t frame_bytes, int pairs,
+                             const uint8_t* cut, void* stream);
 /* scipy.ndimage.gaussian_filter(x, sigma) on N maps [N,H,W] (truncate 4, mode 'reflect';
  * src/fusion_net/interpolate_twoframe.py:212-213).  tmp: scratch of the same size. */
 int fvfi_gaussian_filter(const float* in, float* out, float* tmp, int N, int H, int W, float sigma, void* stream);
